@@ -2,6 +2,7 @@
 """bench.py -- encode+decode throughput of the batched rANS / float codec.
 
     python bench.py --gpus N --steps K --warmup W [--impl ours|reference] [--workload c3|c2|c4|c3x1]
+                    [--dump-outputs DIR]
 
 A "step" = one pass of the hot path over one batch: compress the whole batch,
 then decompress it.  metric = uncompressed GB/s through encode+decode
@@ -40,6 +41,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the source tree may be read-only; the bench writes nothing into it
 
 MIB = 1 << 20
 WORKLOADS = {
@@ -301,6 +303,39 @@ class RefGpuCodec:
     launches_per_step = 0
 
 
+DUMP_SAMPLES = 4 * MIB  # values sampled from the archives and from the decoded batch: 2 x 16 MiB of float32
+
+
+def dump_outputs(out_dir, torch, codec, kind):
+    """Writes what the last codec step returned to its caller, so that two builds can be compared on the
+    same inputs: the compressed sizes (float64) and a fixed, seeded sample of the archives and of the
+    decoded batch (float32, both exact).  The format leaves some archive bytes free (where each block's
+    stream sits in the data section, padding), and they differ from run to run, so each archive is first
+    reduced to its defined fields in a fixed order (oracle.defined_fields).  Sample positions are drawn over
+    the whole row width, which depends on the input sizes only; a position past that reduced archive reads -1."""
+    import numpy as np
+
+    from oracle import oracle as O
+
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(2024)
+    n, cols = codec.comp.shape
+    k = DUMP_SAMPLES // n
+    hs = codec.sizes.cpu().tolist()
+    ft = {"bf16": O.BF16, "f16": O.F16}.get(kind, 0)
+    arch = np.full((n, k), -1, np.float32)
+    for i, h in enumerate(hs):
+        fields = O.defined_fields(codec.comp[i, :h].cpu().numpy(), ft)
+        canon = np.frombuffer(b"".join(fields.values()), np.uint8)
+        pos = np.sort(rng.integers(0, cols, k))
+        inside = pos < canon.size
+        arch[i, inside] = canon[pos[inside]]
+    dec = [o[torch.from_numpy(np.sort(rng.integers(0, o.numel(), k))).to(o.device)].float() for o in codec.outs]
+    np.save(os.path.join(out_dir, "compressed_sizes.npy"), np.array(hs, np.float64))
+    np.save(os.path.join(out_dir, "compressed_sample.npy"), arch)
+    np.save(os.path.join(out_dir, "decompressed_sample.npy"), torch.stack(dec).cpu().numpy())
+
+
 def cpu_baseline(kind, batch, per, budget_s=12.0, pb=10):
     """Oracle port on the host cores, bounded sample of the same workload.  One C call takes the whole
     sample batch and spreads split / histogram / block coding / packing (and the inverse) over all
@@ -358,6 +393,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--all-workloads", action="store_true", help="(default now; kept for old command lines)")
     ap.add_argument("--no-detail", action="store_true", help="skip the short runs of the other BASELINE workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0: compressed sizes, a seeded "
+                         "sample of the archives and of the decoded batch) to DIR/<name>.npy; inputs are seeded, so "
+                         "runs with the same arguments can be compared")
     args = ap.parse_args()
 
     import torch
@@ -380,6 +419,8 @@ def main():
     use_ref_gpu = args.impl == "reference" and ref_lib.available()
     if args.impl == "reference" and not use_ref_gpu:
         # no compiled reference here: the reference arm is the CPU port
+        if args.dump_outputs:
+            ap.error("--dump-outputs: the CPU port that stands in for a missing reference build has no outputs to dump")
         if rank == 0:
             kind, batch, per, desc = WORKLOADS[args.workload]
             cb = cpu_baseline(kind, batch, per, budget_s=60.0, pb=PROB_BITS.get(args.workload, 10))
@@ -456,6 +497,8 @@ def main():
             "value": world * 2 * ubytes * steps / t_tot / 1e9, "clocks": clocks, "cbytes_all": cbytes_all,
             "launches": launches, "prob_bits": pb,
         }
+        if full and args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, torch, codec, kind)
         if not full:
             return res
 

@@ -9,9 +9,9 @@
  * CUDA library is missing instead of falling back here.
  *
  * Parity pin: the restatement is checked (tests/test_oracle.py) against the
- * reference's own known-answer tests (ANSStatisticsTest.cu:127-167) and, on a
- * GPU box, against the reference itself compiled for sm_100a into oracle/_ref/
- * (tests/test_reference_parity.py).
+ * reference's own known-answer tests (ANSStatisticsTest.cu:127-167) and against
+ * archives written by the reference itself, compiled for sm_100a
+ * (tests/golden/ref_golden.npz, tests/test_reference_parity.py).
  *
  * Every function cites the reference file:line (relative to
  * /root/reference/dietgpu/) whose behaviour it restates.  The text below is a

@@ -255,6 +255,32 @@ def assert_same_ans(mine, ref, what: str = "") -> None:
         assert np.array_equal(x, y), f"{what}: stream of block {i}"
 
 
+def defined_fields(arch, ft: int = 0) -> dict:
+    """The parts of an archive that the format defines, as bytes, under stable names: exactly what
+    assert_same_ans (ft = 0, a raw-byte archive) or the float comparison of the parity tests looks at.
+    Streams are concatenated in block order, so their placement inside the data section does not count.
+    Stored as digests, these let an archive be compared with one that is too large to keep."""
+    a = _bytes(arch)
+    out = {}
+    if ft:
+        n = int(a[4:8].view(np.uint32)[0])
+        out["float_header"] = bytes(a[:8]) + bytes([int(a[8]) & 0x1F]) + bytes(a[12:16])
+        if ft == F32:
+            o1 = 16 + 2 * ((n + 7) // 8 * 8)
+            out["float_planes"] = bytes(a[16:16 + 2 * n]) + bytes(a[o1:o1 + n])
+        else:
+            out["float_planes"] = bytes(a[16:16 + n])
+        a = a[16 + float_noncomp_bytes(ft, n):]
+    p = parse_ans(a)
+    hdr = [p[k] for k in ("magic", "num_blocks", "uncompressed", "total_words", "prob_bits", "use_checksum", "size")]
+    out["ans_header"] = np.array(hdr + [p["checksum"] if p["use_checksum"] else 0], np.uint32).tobytes()
+    out["pdf"] = p["pdf"].tobytes()
+    out["states"] = p["states"].tobytes()
+    out["block_sizes"] = p["block_words"][:, 0].tobytes()
+    out["streams"] = b"".join(s.tobytes() for s in p["streams"])
+    return out
+
+
 def assert_same_float(mine, ref, ft: int, what: str = "") -> None:
     """Float archives: header and stored planes byte-equal, ANS part semantically equal."""
     m, r = _bytes(mine), _bytes(ref)

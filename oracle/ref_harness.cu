@@ -1,7 +1,7 @@
 // ref_harness.cu -- TEST INFRASTRUCTURE ONLY (written for this repo).
 // A C-ABI veneer over the UNMODIFIED reference library so Python (ctypes) can
 // drive the reference's own CUDA path: as the GPU-side parity oracle
-// (tests/test_reference_parity.py) and as the `--impl reference` arm of
+// (tests/golden/make_ref_golden.py) and as the `--impl reference` arm of
 // bench.py.  It is compiled together with the reference sources, where they
 // lie under /root/reference, by build_ref.sh into oracle/_ref/ (git-ignored).
 // No reference source is copied into this repository.

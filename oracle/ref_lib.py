@@ -1,7 +1,7 @@
 """ctypes binding of oracle/_ref/libdietgpu_ref.so -- the UNMODIFIED reference
 (facebookresearch/dietgpu) compiled for sm_100a by oracle/build_ref.sh, behind
 the C veneer oracle/ref_harness.cu.  TEST / BASELINE infrastructure only: used
-by tests/test_reference_parity.py and by `bench.py --impl reference`.
+by tests/golden/make_ref_golden.py and by `bench.py --impl reference`.
 """
 from __future__ import annotations
 

@@ -1,20 +1,24 @@
 """The reference's OWN googletest suites (dietgpu/ans/ANSTest.cu:243-282, dietgpu/float/FloatTest.cu:
-270-311), compiled unchanged from /root/reference against libdietgpu_b200.so through the include-path
-shim tests/ref_shim -> include/dietgpu_b200_compat.hpp (tests/cpp/build_ref_tests.sh, run by
-__graft_entry__.build() in the container that has the reference; the binaries travel to the GPU box).
-SURVEY.md section 8f-1's acceptance line: ANSTest and FloatTest pass against the new library."""
+270-311), compiled unchanged against libdietgpu_b200.so through the include-path shim tests/ref_shim ->
+include/dietgpu_b200_compat.hpp.  SURVEY.md section 8f-1's acceptance line: ANSTest and FloatTest pass
+against the new library.
+
+Their sources belong to the reference and are not part of this repository: `oracle/build_ref.sh gtests`,
+run by __graft_entry__.build() where the reference's sources are present, compiles them into oracle/_ref/,
+and a missing binary is a failure here.  The same cases, written for this repository, also run through
+tests/test_gpu_compat.py."""
 import os
 import subprocess
 
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
+REF_BIN = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref")
 
 
 def _run(name, expect_tests):
-    exe = os.path.join(HERE, "cpp", name)
+    exe = os.path.join(REF_BIN, name)
     if not os.path.exists(exe):
-        pytest.fail(f"{exe} missing: run tests/cpp/build_ref_tests.sh where /root/reference exists")
+        pytest.fail(f"{exe} missing: `oracle/build_ref.sh gtests` builds it where the reference's sources are present")
     p = subprocess.run([exe, "--gtest_color=no"], capture_output=True, text=True, timeout=900)
     out = p.stdout + p.stderr
     assert p.returncode == 0, out[-4000:]
