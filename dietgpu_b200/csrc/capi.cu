@@ -86,15 +86,9 @@ void splitParts(const uint64_t* weight, uint32_t n, int parts, uint32_t* bounds)
   bounds[0] = 0;
   uint64_t acc = 0;
   uint32_t idx = 0;
-  // options first_part_pct / last_part_pct: size of the first / last sub-batch in percent of an equal share
-  // (100 = equal); the middle sub-batches share the rest equally
-  const int fp = parts > 2 ? std::max(10, std::min(200, options().first_part_pct)) : 100;
-  const int lp = parts > 2 ? std::max(10, std::min(200, options().last_part_pct)) : 100;
   const uint64_t eq = total / (uint64_t)parts;
-  const uint64_t first = eq * (uint64_t)fp / 100u, last = eq * (uint64_t)lp / 100u;
-  const uint64_t mid = parts > 2 && total > first + last ? (total - first - last) / (uint64_t)(parts - 2) : eq;
   for (int p = 1; p < parts; ++p) {
-    const uint64_t target = (parts > 2 && (fp != 100 || lp != 100)) ? first + mid * (uint64_t)(p - 1) : eq * (uint64_t)p;
+    const uint64_t target = eq * (uint64_t)p;
     const uint32_t mustLeave = (uint32_t)(parts - p);  // one member for every later part
     while (idx + mustLeave < n && (idx < bounds[p - 1] + 1 || acc + weight[idx] / 2 <= target)) acc += weight[idx++];
     bounds[p] = idx;
@@ -102,14 +96,13 @@ void splitParts(const uint64_t* weight, uint32_t n, int parts, uint32_t* bounds)
   bounds[parts] = n;
 }
 
-int autoParts(int kind, uint32_t n, uint64_t totalBytes, bool decode) {
+int autoParts(int kind, uint32_t n, uint64_t totalBytes) {
   const Options& o = options();
   if (o.timing) return 1;  // per-kernel timing wants un-overlapped launches
   int p = o.parts;
   // measured on B200 (tools/walltime.py, 256 MiB batches): float encode is best with 4 sub-batches
   // (the bandwidth-bound statistics kernel of one sub-batch runs beside the issue-bound coder of the
-  // previous one: c3 204 / 195 / 189 us for 1 / 2 / 4), the two-kernel decoder with 4 (plan latency
-  // and kernel tails hide); byte inputs gain nothing
+  // previous one: c3 204 / 195 / 189 us for 1 / 2 / 4); byte inputs gain nothing
   if (p <= 0) {
     const bool big = kind != kKindBytes && totalBytes >= (64ull << 20);
     p = !big ? 1 : (n >= 16 ? 4 : (n >= 8 ? 2 : 1));
@@ -393,26 +386,16 @@ int dgb_archives_pull(int float_type, uint32_t num_in_batch, const void* const* 
 
 static int* optionSlot(Options& o, const char* name) {
   if (!name) return nullptr;
-  if (!std::strcmp(name, "decode_fused")) return &o.decode_fused;
   if (!std::strcmp(name, "decode_warps")) return &o.decode_warps;
   if (!std::strcmp(name, "decode_slot_words")) return &o.decode_slot_words;
   if (!std::strcmp(name, "encode_warps")) return &o.encode_warps;
   if (!std::strcmp(name, "encode_canonical")) return &o.encode_canonical;
-  if (!std::strcmp(name, "encode_fused")) return &o.encode_fused;
-  if (!std::strcmp(name, "fused_stats_every")) return &o.fused_stats_every;
-  if (!std::strcmp(name, "fused_stage")) return &o.fused_stage;
-  if (!std::strcmp(name, "fused_chunk_blocks")) return &o.fused_chunk_blocks;
   if (!std::strcmp(name, "encode_wide_table")) return &o.encode_wide_table;
   if (!std::strcmp(name, "encode_slot_words")) return &o.encode_slot_words;
-  if (!std::strcmp(name, "stats_stage")) return &o.stats_stage;
-  if (!std::strcmp(name, "stats_stage_kb")) return &o.stats_stage_kb;
-  if (!std::strcmp(name, "encode_k2_ctas")) return &o.encode_k2_ctas;
   if (!std::strcmp(name, "hist_slab_kb")) return &o.hist_slab_kb;
   if (!std::strcmp(name, "hist_ctas_per_sm")) return &o.hist_ctas_per_sm;
   if (!std::strcmp(name, "inline_members")) return &o.inline_members;
   if (!std::strcmp(name, "pull_ctas")) return &o.pull_ctas;
-  if (!std::strcmp(name, "first_part_pct")) return &o.first_part_pct;
-  if (!std::strcmp(name, "last_part_pct")) return &o.last_part_pct;
   if (!std::strcmp(name, "timing")) return &o.timing;
   if (!std::strcmp(name, "parts")) return &o.parts;
   return nullptr;
@@ -442,7 +425,8 @@ int dgb_clear_thread_options(void) {
 }
 
 // Sum of the event-timed durations (ms) and launch counts per kernel slot since the last
-// call; synchronises the device.  Slots: 0 stats(K1) 1 encode(K2) 2 plan 3 decode 4 checksum.
+// call; synchronises the device.  Slots: 0 stats(K1) 1 encode(K2) 3 decode 4 checksum 6 archive mover
+// (2 and 5 are retired and always 0).
 int dgb_kernel_times(float* ms, int* counts, int nslots) {
   if (cudaDeviceSynchronize() != cudaSuccess) return DGB_ERR_CUDA;
   std::lock_guard<std::mutex> lock(timerMutex());
@@ -459,7 +443,7 @@ int dgb_kernel_times(float* ms, int* counts, int nslots) {
 }
 
 int dgb_get_option(const char* name, int* value) {
-  // read-only counter: hot-path kernels launched so far (stats, encode, plan, decode)
+  // read-only counter: hot-path kernels launched so far (stats, encode, decode, archive mover)
   if (name && value && !std::strcmp(name, "launches")) {
     *value = dgb::gLaunches.load(std::memory_order_relaxed);
     return DGB_OK;

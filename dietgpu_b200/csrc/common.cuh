@@ -8,6 +8,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
+
 #include "../../include/dietgpu_b200.h"
 
 namespace dgb {
@@ -49,15 +51,15 @@ struct MemberDesc {
   const void* in;     // encode: raw input (bytes / float words); decode: archive
   void* out;          // encode: archive; decode: output
   uint32_t size;      // encode: input size (bytes, or float WORDS); decode: capacity (same unit)
-  uint32_t work0;     // first flat work item (chunk / ticket) of this member
+  uint32_t work0;     // encode: first flat 4 KiB block of this member; decode: bound on its block count
 };
 static_assert(sizeof(MemberDesc) == 24, "");
 
 // Batches of up to kInlineMembers members travel to the default kernels INSIDE the kernel parameters
 // (constant bank, 1.5 KB) instead of through a host-to-device copy in front of the first launch: one
 // dependent DMA less per call, nothing of the caller's host memory is read after the call returns,
-// and the whole call can be captured into a CUDA graph.  Larger batches (and the optional kernel
-// flavours) read the same table from the scratch buffer.
+// and the whole call can be captured into a CUDA graph.  Larger batches (and the canonical encoder)
+// read the same table from the scratch buffer.
 constexpr uint32_t kInlineMembers = 64;
 struct InlineMembers {
   uint32_t count;  // 0: the table is in global memory (scratch)
@@ -89,25 +91,15 @@ struct __align__(16) EncEntryWide {
 
 // ---- tuning options (dgb_set_option) ---------------------------------------
 struct Options {
-  int decode_fused = 1;      // 1: one persistent launch, CTAs lease members and warps claim blocks; 0: plan + decode kernels
-  int decode_warps = 0;      // single-launch decoder: warps per CTA (4, 8, 20 = byte archives only; 0 = auto)
+  int decode_warps = 0;      // decoder warps per CTA: 8, or 20 for byte archives; 0 = auto
   int decode_slot_words = 0; // TMA staging slot per warp in u16 words; 0 = auto
   int encode_warps = 8;      // warps per encode CTA (each warp is an independent worker)
   int encode_slot_words = 0; // staging slot of the fast encoder in u16 words; 0 = auto
   int encode_canonical = 0;  // 1: streams packed in block order (byte-identical archives, slower)
-  int encode_fused = 0;      // 1: one persistent launch (statistics items + encode chunks), 0: two kernels (default: measured equal or faster)
-  int fused_stage = 1;       // fused launch: statistics slabs land in shared memory by TMA bulk copy (0: register loads)
-  int fused_stats_every = 4; // fused launch: one CTA in this many prefers statistics items (0: none does)
-  int fused_chunk_blocks = 16;  // fused launch: 4 KiB blocks per encode chunk
   int encode_wide_table = -1;  // encoder table entries: 1 = 16 B, 0 = 8 B, -1 = by data kind (bf16/fp32 wide)
-  int stats_stage = 0;       // two-kernel path, float kinds: 1 = statistics slab lands in shared memory by TMA (one slab per CTA)
-  int stats_stage_kb = 32;   // ... slab size for that
-  int encode_k2_ctas = 0;    // cap of coder CTAs per SM (0 = as many as fit)
   int hist_slab_kb = 64;     // bytes of input per histogram CTA iteration
   int hist_ctas_per_sm = 32; // stats grid = this many CTAs per SM (each CTA loops over slabs)
-  int parts = 0;             // sub-batches run on internal streams (0 = auto, 1 = off, max 4)
-  int first_part_pct = 100;  // size of the first / last sub-batch relative to an equal share (capi.cu splitParts)
-  int last_part_pct = 100;
+  int parts = 0;             // encode sub-batches run on internal streams (0 = auto, 1 = off, max 8)
   int pull_ctas = 64;        // grid of the archive mover (dgb_archives_pull): enough loads in flight for NVLink, few SMs
   int inline_members = 1;   // 1: member table inside the kernel parameters when the batch has <= 64 members
   int timing = 0;            // 1: bracket every kernel launch with CUDA events (bench.py roofline pass)
@@ -138,11 +130,12 @@ int pullArchives(int kind, uint32_t n, const void* const* src, void* const* dst,
 void setLastCudaError(cudaError_t e);
 
 // Per-kernel timing (options().timing): slots are stable indices reported by
-// dgb_kernel_times().  No-ops when timing is off.
-enum TimerSlot : int { kSlotStats = 0, kSlotEncode = 1, kSlotPlan = 2, kSlotDecode = 3, kSlotChecksum = 4, kSlotFused = 5, kSlotPull = 6, kNumSlots = 7 };
-// Internal helper streams: a large batch is cut into up to kMaxParts contiguous sub-batches whose
+// dgb_kernel_times() (C ABI).  Slots 2 and 5 are retired and always report 0.
+// No-ops when timing is off.
+enum TimerSlot : int { kSlotStats = 0, kSlotEncode = 1, kSlotDecode = 3, kSlotChecksum = 4, kSlotPull = 6, kNumSlots = 7 };
+// Internal helper streams: a large encode batch is cut into up to kMaxParts contiguous sub-batches whose
 // kernels run on separate streams (forked from / joined to the caller's stream with events), so the
-// HBM-bound and the issue-bound kernels of different sub-batches overlap and launch gaps hide.
+// HBM-bound statistics kernel of one sub-batch overlaps the issue-bound coder of another.
 constexpr int kMaxParts = 8;
 struct StreamPool {
   cudaStream_t s[kMaxParts];
@@ -151,7 +144,7 @@ struct StreamPool {
 int streamPool(StreamPool** out);  // lazily created; DGB_OK or DGB_ERR_CUDA
 // cuts members [0,n) into `parts` contiguous ranges of roughly equal `weight`; bounds has parts+1 entries
 void splitParts(const uint64_t* weight, uint32_t n, int parts, uint32_t* bounds);
-int autoParts(int kind, uint32_t n, uint64_t totalBytes, bool decode);
+int autoParts(int kind, uint32_t n, uint64_t totalBytes);
 
 void timerBegin(int slot, cudaStream_t stream);
 void timerEnd(int slot, cudaStream_t stream);
@@ -164,6 +157,42 @@ void timerEnd(int slot, cudaStream_t stream);
       return DGB_ERR_CUDA;                    \
     }                                         \
   } while (0)
+
+inline size_t alignUp256(size_t v) { return (v + 255) & ~size_t(255); }
+
+// SMs of the current device, cached per device (a process may drive several); racing first calls
+// write the same value
+inline int smCount() {
+  static int cached[64] = {};
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
+  if (!cached[dev]) {
+    int v = 0;
+    cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
+    cached[dev] = v > 0 ? v : 148;
+  }
+  return cached[dev];
+}
+
+// CTAs of KERN that fit on one SM with `threads` threads and `smemBytes` of dynamic shared memory
+// (at least 1).  Cached per host thread and kernel; queried again when the block size, the shared
+// memory or the current device changes (function attributes are per device).
+template <auto KERN>
+int residentPerSm(int threads, size_t smemBytes, int maxSmemBytes, int* out) {
+  static thread_local int perSm = 0, keyThreads = 0, keyDev = -1;
+  static thread_local size_t keySmem = 0;
+  int dev = 0;
+  DGB_CUDA_TRY(cudaGetDevice(&dev));
+  if (perSm == 0 || keyThreads != threads || keySmem != smemBytes || keyDev != dev) {
+    DGB_CUDA_TRY(cudaFuncSetAttribute(KERN, cudaFuncAttributeMaxDynamicSharedMemorySize, maxSmemBytes));
+    int occ = 0;
+    DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, KERN, threads, smemBytes));
+    perSm = std::max(occ, 1);
+    keyThreads = threads; keySmem = smemBytes; keyDev = dev;
+  }
+  *out = perSm;
+  return DGB_OK;
+}
 
 #ifdef __CUDACC__
 // ---- small device helpers ---------------------------------------------------
@@ -222,6 +251,22 @@ __device__ __forceinline__ void bulkLoad(uint32_t dstSmem, const void* src, uint
       "l"(src), "r"(bytes), "r"(bar)
       : "memory");
 }
+// ---- cp.async (LDGSTS): 16 B global -> shared copies in commit groups --------
+__device__ __forceinline__ void cpAsync16(uint32_t dstSmem, const void* src) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dstSmem), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cpAsyncCommit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cpAsyncWait() {
+  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
+}
+template <int OFF>
+__device__ __forceinline__ uint32_t ldsU8(uint32_t addr) {
+  uint32_t v;
+  asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(OFF));
+  return v;
+}
+
 // block-wide exclusive scan of one value per thread for THREADS threads
 // (THREADS multiple of 32, <= 1024).  `warpSums` is smem of THREADS/32 words.
 template <int THREADS>

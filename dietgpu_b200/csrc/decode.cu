@@ -6,9 +6,8 @@
 // runs with table look-ups and the loop-carried refill load in shared memory, and float kinds join the
 // decoded byte with the stored byte(s) (cp.async ring) and store the float word in the same loop, at any
 // alignment (float/GpuFloatDecompress.cuh:22-179, float/GpuFloatUtils.cuh:100-204 join rules; the
-// reference's two-pass path, float/GpuFloatDecompress.cuh:622-694, is not needed).
-// The round-1 pair planKernel (header validation ans/GpuANSDecode.cuh:326-341, flat block offsets) +
-// decodeKernel (static split of the blocks) is kept behind option decode_fused=0.
+// reference's two-pass path, float/GpuFloatDecompress.cuh:622-694, is not needed).  A batch is never
+// cut into sub-batches: the persistent grid already balances the blocks of every member.
 #include <algorithm>
 #include <cstring>
 #include <vector>
@@ -28,11 +27,9 @@ namespace dgb {
 namespace {
 
 struct DecodeScratch {
-  MemberDesc* members;   // [n]; two-kernel path: planKernel fills work0 = first flat block;
-                         //      single-launch path: work0 = upper bound of the member's block count (host, from capacity)
-  uint32_t* next;        // [n] single-launch path: next unclaimed block of the member (zeroed)
-  uint32_t* seen;        // [n] single-launch path: 1 once a CTA has reported the member (zeroed)
-  uint32_t* totals;      // [0] = total blocks, [1] = unused
+  MemberDesc* members;   // [n]; work0 = upper bound of the member's block count (host, from capacity)
+  uint32_t* next;        // [n] next unclaimed block of the member (zeroed)
+  uint32_t* seen;        // [n] 1 once a CTA has reported the member (zeroed)
   uint32_t* checksum;    // [n] checksum of decoded output (use_checksum only; zeroed)
   uint32_t* archiveChecksum;  // [n]
   uint32_t* sizes;       // [n] decoded size in bytes (for the checksum pass)
@@ -66,54 +63,6 @@ __device__ __forceinline__ ArchiveView openArchive(const uint8_t* in) {
 }
 
 // ---------------------------------------------------------------------------
-// P: plan.  One CTA; member i handled by thread (i % blockDim) in rounds.
-// ---------------------------------------------------------------------------
-template <int KIND>
-__global__ void __launch_bounds__(1024)
-planKernel(DecodeScratch sc, uint32_t m0, uint32_t m1, uint32_t part, int pb,
-           uint8_t* __restrict__ outSuccess, uint32_t* __restrict__ outSize, bool wantChecksum) {
-  // members [m0, m1) form one sub-batch with its own flat block index space (totals[part])
-  __shared__ uint32_t sWarp[32];
-  uint32_t carry = 0;
-  const uint32_t n = m1;
-  for (uint32_t base = m0; base < n; base += blockDim.x) {
-    const uint32_t i = base + threadIdx.x;
-    uint32_t blocks = 0;
-    if (i < n) {
-      const MemberDesc md = sc.members[i];
-      const ArchiveView av = openArchive<KIND>(static_cast<const uint8_t*>(md.in));
-      bool ok = av.ok;
-      uint32_t need = 0, nb = 0, storedChecksum = 0;
-      if (ok) {
-        const uint4 h0 = __ldg(reinterpret_cast<const uint4*>(av.ans));
-        const uint4 h1 = __ldg(reinterpret_cast<const uint4*>(av.ans) + 1);
-        nb = h0.y;
-        need = h0.z;  // uncompressed bytes == float words for float kinds
-        ok = h0.x == kAnsMagicVersion && (int)(h1.x & 0xfu) == pb && nb == divUp(need, kBlockBytes);
-        if (KIND != kKindBytes) ok = ok && need == av.floatWords;
-        storedChecksum = KIND == kKindBytes
-            ? h1.y
-            : __ldg(reinterpret_cast<const uint32_t*>(md.in) + 3);
-      }
-      // ans/GpuANSDecode.cuh:326-337: success iff capacity suffices; size reported regardless
-      const bool success = ok && md.size >= need;
-      if (outSuccess) outSuccess[i] = success ? 1 : 0;
-      if (outSize) outSize[i] = ok ? need : 0u;
-      if (wantChecksum) {
-        sc.archiveChecksum[i] = storedChecksum;
-        sc.sizes[i] = success ? need : 0u;
-      }
-      blocks = success ? nb : 0u;
-    }
-    uint32_t tot;
-    const uint32_t excl = blockExclusiveScan<1024>(blocks, sWarp, &tot);
-    if (i < n) sc.members[i].work0 = carry + excl;
-    carry += tot;
-  }
-  if (threadIdx.x == 0) sc.totals[part] = carry;
-}
-
-// ---------------------------------------------------------------------------
 // Output writers (ans/BatchProvider.cuh:16-37 BatchWriter, float/
 // GpuFloatDecompress.cuh:391-486 JoinFloatWriter restated).  A writer is bound
 // to one 4 KiB block.  The float kinds need the stored ("non-compressed")
@@ -131,20 +80,6 @@ planKernel(DecodeScratch sc, uint32_t m0, uint32_t m1, uint32_t part, int pb,
 constexpr int kGroupRows = DGB_DEC_GROUP_ROWS;  // rows per prefetch group (8 or 16)
 constexpr uint32_t kRingSlots = 3;              // groups resident per warp: current + 2 in flight
 
-__device__ __forceinline__ void cpAsync16(uint32_t dstSmem, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dstSmem), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cpAsyncCommit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cpAsyncWait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-template <int OFF>
-__device__ __forceinline__ uint32_t ldsU8(uint32_t addr) {
-  uint32_t v;
-  asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(OFF));
-  return v;
-}
 template <int OFF>
 __device__ __forceinline__ uint32_t ldsU16(uint32_t addr) {
   uint32_t v;
@@ -293,17 +228,15 @@ struct GmemStream {
 };
 
 // ---------------------------------------------------------------------------
-// Decode LUT, one entry per state residue (never leaves shared memory):
-//   LUT64 = false: u32  [31:20] pdf  [19:8] s-cdf  [7:0] symbol
-//   LUT64 = true : uint2 {pdf, (s-cdf) << 8 | symbol}   -- two fewer ALU ops per
-//                  row for the unpack, twice the shared-memory footprint
+// Decode LUT, one u32 entry per state residue (never leaves shared memory):
+//   [31:20] pdf  [19:8] s-cdf  [7:0] symbol
+// (8-byte entries {pdf, (s-cdf) << 8 | symbol} save two ALU ops per row for the unpack, take twice
+// the shared memory, and measured slower on every workload.)
 // One decode step for a full row (ans/GpuANSDecode.cuh:55-105 restated); the
 // returned word has the decoded symbol in its low byte.
 // ---------------------------------------------------------------------------
-template <int PB, bool LUT64>
-struct Lut;
 template <int PB>
-struct Lut<PB, false> {
+struct Lut {
   typedef uint32_t Entry;
   static __device__ __forceinline__ Entry make(uint32_t pdf, uint32_t c, uint32_t sym) {
     return (pdf << 20) | (c << 8) | sym;
@@ -314,18 +247,6 @@ struct Lut<PB, false> {
     // (s - cdf) field needs no mask (all arithmetic mod 2^32); the -4096 folds into the shift (LEA.HI)
     state = (e >> 20) * ((state >> PB) - 4096u) + (e >> 8);
     return e;
-  }
-};
-template <int PB>
-struct Lut<PB, true> {
-  typedef uint2 Entry;
-  static __device__ __forceinline__ Entry make(uint32_t pdf, uint32_t c, uint32_t sym) {
-    return make_uint2(pdf, (c << 8) | sym);
-  }
-  static __device__ __forceinline__ uint32_t step(uint32_t& state, const Entry* __restrict__ lut) {
-    const uint2 e = lut[state & ((1u << PB) - 1u)];
-    state = e.x * (state >> PB) + (e.y >> 8);
-    return e.y;
   }
 };
 
@@ -365,21 +286,21 @@ __device__ __forceinline__ void refill<SmemStream>(uint32_t& state, SmemStream& 
       : "r"(geMask));
 }
 
-template <int PB, bool LUT64, typename Stream>
+template <int PB, typename Stream>
 __device__ __forceinline__ uint32_t decodeStep(uint32_t& state,
-                                               const typename Lut<PB, LUT64>::Entry* __restrict__ lut,
+                                               const typename Lut<PB>::Entry* __restrict__ lut,
                                                Stream& st, uint32_t geMask) {
-  const uint32_t e = Lut<PB, LUT64>::step(state, lut);
+  const uint32_t e = Lut<PB>::step(state, lut);
   refill(state, st, geMask);
   return e;
 }
 
-template <int PB, bool LUT64, typename Stream>
+template <int PB, typename Stream>
 __device__ __forceinline__ uint32_t decodeStepPartial(bool valid, uint32_t& state,
-                                                      const typename Lut<PB, LUT64>::Entry* __restrict__ lut,
+                                                      const typename Lut<PB>::Entry* __restrict__ lut,
                                                       Stream& st, uint32_t geMask) {
   uint32_t s2 = state;
-  const uint32_t e = Lut<PB, LUT64>::step(s2, lut);
+  const uint32_t e = Lut<PB>::step(s2, lut);
   if (valid) state = s2;
   const bool rd = valid && state < kStateMin;
   const uint32_t vote = __ballot_sync(0xffffffffu, rd);
@@ -388,33 +309,33 @@ __device__ __forceinline__ uint32_t decodeStepPartial(bool valid, uint32_t& stat
   return e;
 }
 
-template <int KIND, int PB, bool LUT64, typename Stream, int J>
+template <int KIND, int PB, typename Stream, int J>
 struct RowGroup {
   typedef RowWriter<KIND> W;
   // rows J-1 .. 0 of the group, highest first (the decoder walks rows backwards)
   static __device__ __forceinline__ void run(uint32_t& state,
-                                             const typename Lut<PB, LUT64>::Entry* __restrict__ lut,
+                                             const typename Lut<PB>::Entry* __restrict__ lut,
                                              Stream& st, uint32_t geMask, const W& wr,
                                              const typename W::Cursor& c) {
-    const uint32_t e = decodeStep<PB, LUT64>(state, lut, st, geMask);
+    const uint32_t e = decodeStep<PB>(state, lut, st, geMask);
     wr.template write<J - 1>(c, e);
-    RowGroup<KIND, PB, LUT64, Stream, J - 1>::run(state, lut, st, geMask, wr, c);
+    RowGroup<KIND, PB, Stream, J - 1>::run(state, lut, st, geMask, wr, c);
   }
 };
-template <int KIND, int PB, bool LUT64, typename Stream>
-struct RowGroup<KIND, PB, LUT64, Stream, 0> {
+template <int KIND, int PB, typename Stream>
+struct RowGroup<KIND, PB, Stream, 0> {
   typedef RowWriter<KIND> W;
-  static __device__ __forceinline__ void run(uint32_t&, const typename Lut<PB, LUT64>::Entry* __restrict__, Stream&,
+  static __device__ __forceinline__ void run(uint32_t&, const typename Lut<PB>::Entry* __restrict__, Stream&,
                                              uint32_t, const W&, const typename W::Cursor&) {}
 };
 
-template <int KIND, int PB, bool LUT64, typename Stream>
+template <int KIND, int PB, typename Stream>
 __device__ __forceinline__ void decodeBlockWarp(uint32_t state, Stream st, uint32_t n,
-                                                const typename Lut<PB, LUT64>::Entry* __restrict__ lut,
+                                                const typename Lut<PB>::Entry* __restrict__ lut,
                                                 const RowWriter<KIND>& wr, uint32_t lane) {
   typedef typename RowWriter<KIND>::Cursor Cursor;
   constexpr int U = kGroupRows;
-  typedef RowGroup<KIND, PB, LUT64, Stream, U> G;
+  typedef RowGroup<KIND, PB, Stream, U> G;
   const uint32_t geMask = laneMaskGe();
   uint32_t row = n >> 5;  // number of full rows; the partial row (if any) has this index
   const uint32_t rem = n & 31u;
@@ -430,7 +351,7 @@ __device__ __forceinline__ void decodeBlockWarp(uint32_t state, Stream st, uint3
   cpAsyncCommit();
   if (rem) {
     const bool valid = lane < rem;
-    const uint32_t e = decodeStepPartial<PB, LUT64>(valid, state, lut, st, geMask);
+    const uint32_t e = decodeStepPartial<PB>(valid, state, lut, st, geMask);
     if (valid) wr.writeSlow(row, e);
   }
   uint32_t slot = 0, slotNext = 2;  // ring slots of group k and of group k + 2
@@ -449,15 +370,15 @@ __device__ __forceinline__ void decodeBlockWarp(uint32_t state, Stream st, uint3
   }
   while (row > 0) {
     --row;
-    const uint32_t e = decodeStep<PB, LUT64>(state, lut, st, geMask);
+    const uint32_t e = decodeStep<PB>(state, lut, st, geMask);
     wr.writeSlow(row, e);
   }
 }
 
 // LUT build from the archive's u16 pdf[256] (ans/GpuANSDecode.cuh:405-476
 // restated; runs inside the decode CTA).  blockDim.x == WARPS*32.
-template <int PB, bool LUT64, int WARPS>
-__device__ void buildLut(const uint8_t* __restrict__ ans, typename Lut<PB, LUT64>::Entry* __restrict__ lut,
+template <int PB, int WARPS>
+__device__ void buildLut(const uint8_t* __restrict__ ans, typename Lut<PB>::Entry* __restrict__ lut,
                          uint32_t* sPdf, uint32_t* sCdf, uint32_t* sWarp) {
   constexpr int T = WARPS * 32;
   constexpr int PER = (kNumSymbols + T - 1) / T;
@@ -484,110 +405,14 @@ __device__ void buildLut(const uint8_t* __restrict__ ans, typename Lut<PB, LUT64
   for (uint32_t sym = warp; sym < kNumSymbols; sym += WARPS) {
     const uint32_t pdf = sPdf[sym], begin = sCdf[sym];
     for (uint32_t j = lane; j < pdf; j += 32u) {
-      if (begin + j < (1u << PB)) lut[begin + j] = Lut<PB, LUT64>::make(pdf, j, sym);
+      if (begin + j < (1u << PB)) lut[begin + j] = Lut<PB>::make(pdf, j, sym);
     }
   }
   __syncthreads();
 }
 
-template <int KIND, int PB, int WARPS, bool STAGE, bool LUT64>
-__global__ void __launch_bounds__(WARPS * 32, DGB_DECODE_WARPS_PER_SM / WARPS)
-decodeKernel(DecodeScratch sc, uint32_t m0, uint32_t m1, uint32_t part, uint32_t slotWords) {
-  extern __shared__ __align__(128) uint8_t smem[];
-  constexpr uint32_t K = 1u << PB;
-  typedef typename Lut<PB, LUT64>::Entry Entry;
-  __shared__ __align__(16) Entry lut[K];  // static: constant base address for the hot LDS
-  uint32_t* sPdf = reinterpret_cast<uint32_t*>(smem);
-  uint32_t* sCdf = sPdf + kNumSymbols;
-  uint32_t* sWarp = sCdf + kNumSymbols;           // 32 words
-  uint32_t* sMisc = sWarp + 32;                   // 32 words
-  unsigned long long* sBar = reinterpret_cast<unsigned long long*>(sMisc + 32);  // [WARPS]
-  uint8_t* sRing = reinterpret_cast<uint8_t*>(sBar + ((WARPS + 1) & ~1));  // [WARPS] stored-byte rings
-  constexpr uint32_t ringBytes = kRingSlots * RowWriter<KIND>::kRingSlotBytes;
-  uint8_t* sSlots = sRing + WARPS * ringBytes;
-  const uint32_t slotBytes = 128u + slotWords * 2u;  // lane states + stream
-
-  const uint32_t t = threadIdx.x, lane = t & 31u;
-  // shuffle makes the warp index provably warp-uniform, so the vote in the hot loop needs no
-  // divergence check (BRA.DIV)
-  const uint32_t warp = __shfl_sync(0xffffffffu, t >> 5, 0);
-  uint8_t* mySlot = sSlots + (size_t)warp * slotBytes;
-  const uint32_t myBar = smemAddr(sBar + warp);
-  uint32_t phase = 0;
-  if (STAGE) {
-    if (lane == 0) mbarInit(myBar, 1);
-    fenceBarrierInit();
-    __syncthreads();
-  }
-
-  const uint32_t total = __ldcg(sc.totals + part);
-  // contiguous, balanced run of flat blocks for this CTA
-  const uint64_t g = gridDim.x;
-  uint32_t cur = (uint32_t)((uint64_t)total * blockIdx.x / g);
-  const uint32_t end = (uint32_t)((uint64_t)total * (blockIdx.x + 1) / g);
-
-  while (cur < end) {
-    // member containing flat block `cur`: the last member whose first block <= cur (members
-    // that contribute no blocks share their successor's start and are skipped by the search)
-    if (t == 0) {
-      uint32_t lo = m0, hi = m1;
-      while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (__ldcg(&sc.members[mid].work0) <= cur) lo = mid; else hi = mid;
-      }
-      sMisc[0] = lo;
-    }
-    __syncthreads();
-    const uint32_t m = sMisc[0];
-    const MemberDesc md = sc.members[m];
-    const ArchiveView av = openArchive<KIND>(static_cast<const uint8_t*>(md.in));
-    const uint4 h0 = __ldg(reinterpret_cast<const uint4*>(av.ans));
-    const uint32_t nb = h0.y;
-    const uint32_t memberFirst = __ldcg(&sc.members[m].work0);
-    const uint32_t memberEnd = min(end, memberFirst + nb);
-    buildLut<PB, LUT64, WARPS>(av.ans, lut, sPdf, sCdf, sWarp);
-
-    const uint8_t* pStates = av.ans + kAnsHeaderBytes + kAnsPdfBytes;
-    const uint2* pBlockWords = reinterpret_cast<const uint2*>(pStates + 128u * (size_t)nb);
-    const uint16_t* pData = reinterpret_cast<const uint16_t*>(
-        reinterpret_cast<const uint8_t*>(pBlockWords) + 8u * (size_t)roundUp(nb, 2u));
-    const bool canStage = STAGE && ((reinterpret_cast<uintptr_t>(av.ans) & 15u) == 0);
-
-    RowWriter<KIND> wr;
-    wr.setRing(smemAddr(sRing + warp * ringBytes), lane);
-    for (uint32_t fb = cur + warp; fb < memberEnd; fb += WARPS) {
-      const uint32_t block = fb - memberFirst;
-      const uint2 bw = __ldg(pBlockWords + block);
-      const uint32_t blockLen = bw.x >> 16, words = bw.x & 0xffffu;
-      const uint16_t* stream = pData + bw.y;
-      wr.setBlock(av, md.out, block, lane);
-      // two call sites on purpose: each knows the address space of the stream
-      if (canStage && words <= slotWords && (bw.y & 7u) == 0u) {
-        const uint32_t streamBytes = roundUp(words, 8u) * 2u;
-        __syncwarp();
-        if (lane == 0) {
-          mbarExpectTx(myBar, 128u + streamBytes);
-          bulkLoad(smemAddr(mySlot), pStates + 128u * (size_t)block, 128u, myBar);
-          if (streamBytes) bulkLoad(smemAddr(mySlot + 128), stream, streamBytes, myBar);
-        }
-        mbarWait(myBar, phase);
-        phase ^= 1u;
-        const uint32_t state = reinterpret_cast<const uint32_t*>(mySlot)[lane];
-        SmemStream st{smemAddr(mySlot + 128) + 2u * words};
-        decodeBlockWarp<KIND, PB, LUT64>(state, st, blockLen, lut, wr, lane);
-      } else {
-        const uint32_t state = __ldg(reinterpret_cast<const uint32_t*>(pStates) + block * 32u + lane);
-        GmemStream st{stream + words};
-        decodeBlockWarp<KIND, PB, LUT64>(state, st, blockLen, lut, wr, lane);
-      }
-    }
-    cur = memberEnd;
-    __syncthreads();  // everyone done with this member's LUT before it is rebuilt
-  }
-}
-
 // ---------------------------------------------------------------------------
-// Single-launch decoder (default).  One persistent grid, no plan kernel, no sub-batches.  The host
+// Single-launch decoder.  One persistent grid, one launch per call.  The host
 // knows every member's capacity, hence an upper bound on its 4 KiB block count (work0; at least one
 // so that every header is visited), and zeroes one claim counter per member.  A CTA LEASES a
 // member: it reads and validates the header(s), builds the decode LUT once, and then each of its
@@ -595,8 +420,8 @@ decodeKernel(DecodeScratch sc, uint32_t m0, uint32_t m1, uint32_t part, uint32_t
 // the current block is decoded, so its latency hides) until none are left; only then do the warps
 // meet at a barrier and the CTA moves on to the next member that still has unclaimed blocks,
 // starting from its home member.  Several CTAs lease the same member at once, so the work balances
-// at block granularity and the kernel has no per-block or per-chunk CTA barrier (the static split
-// of the two-kernel path left SMs idle for ~15 % of the kernel, ncu r01).  The first CTA to lease a
+// at block granularity and the kernel has no per-block or per-chunk CTA barrier (a static split of
+// the flat blocks over the CTAs left SMs idle for ~15 % of the kernel, ncu r01).  The first CTA to lease a
 // member reports outSuccess / outSize (ans/GpuANSDecode.cuh:326-341 semantics); claims past the
 // archive's real block count, or of a member that failed, are dropped.
 // Measured and rejected (profiles/r02_wall_experiments.txt, step L): a variant without the lease-end
@@ -613,7 +438,7 @@ decodeFusedKernel(DecodeScratch sc, const __grid_constant__ InlineMembers im, ui
                   uint8_t* __restrict__ outSuccess, uint32_t* __restrict__ outSize, bool wantChecksum) {
   extern __shared__ __align__(128) uint8_t smem[];
   constexpr uint32_t K = 1u << PB;
-  typedef typename Lut<PB, false>::Entry Entry;
+  typedef typename Lut<PB>::Entry Entry;
   __shared__ __align__(16) Entry lut[K];  // static: constant base address for the hot LDS
   uint32_t* sPdf = reinterpret_cast<uint32_t*>(smem);
   uint32_t* sCdf = sPdf + kNumSymbols;
@@ -701,7 +526,7 @@ decodeFusedKernel(DecodeScratch sc, const __grid_constant__ InlineMembers im, ui
       }
     }
     const bool work = memberOk && nb > 0;
-    if (work) buildLut<PB, false, WARPS>(av.ans, lut, sPdf, sCdf, sWarp);
+    if (work) buildLut<PB, WARPS>(av.ans, lut, sPdf, sCdf, sWarp);
 
     const uint8_t* pStates = av.ans + kAnsHeaderBytes + kAnsPdfBytes;
     const uint2* pBlockWords = reinterpret_cast<const uint2*>(pStates + 128u * (size_t)nb);
@@ -738,11 +563,11 @@ decodeFusedKernel(DecodeScratch sc, const __grid_constant__ InlineMembers im, ui
           phase ^= 1u;
           const uint32_t state = reinterpret_cast<const uint32_t*>(mySlot)[lane];
           SmemStream st{smemAddr(mySlot + 128) + 2u * words};
-          decodeBlockWarp<KIND, PB, false>(state, st, blockLen, lut, wr, lane);
+          decodeBlockWarp<KIND, PB>(state, st, blockLen, lut, wr, lane);
         } else {
           const uint32_t state = __ldg(reinterpret_cast<const uint32_t*>(pStates) + block * 32u + lane);
           GmemStream st{stream + words};
-          decodeBlockWarp<KIND, PB, false>(state, st, blockLen, lut, wr, lane);
+          decodeBlockWarp<KIND, PB>(state, st, blockLen, lut, wr, lane);
         }
       }
       block = __shfl_sync(0xffffffffu, nextBlock, 0);
@@ -766,10 +591,8 @@ checksumKernel(DecodeScratch sc) {
   if ((threadIdx.x & 31) == 0 && x) atomicXor(sc.checksum + m, x & 0xffu);
 }
 
-size_t alignUp256(size_t v) { return (v + 255) & ~size_t(255); }
-
 struct DecodePlan {
-  size_t members, next, totals, checksum, archiveChecksum, sizes, total;
+  size_t members, next, checksum, archiveChecksum, sizes, total;
 };
 
 DecodePlan planDecodeScratch(uint32_t n) {
@@ -777,78 +600,11 @@ DecodePlan planDecodeScratch(uint32_t n) {
   size_t o = 0;
   p.members = o; o = alignUp256(o + sizeof(MemberDesc) * (size_t)n);
   p.next = o; o = alignUp256(o + 8 * (size_t)n);  // next[n] then seen[n]
-  p.totals = o; o = alignUp256(o + 4 * kMaxParts);
   p.checksum = o; o = alignUp256(o + 4 * (size_t)n);
   p.archiveChecksum = o; o = alignUp256(o + 4 * (size_t)n);
   p.sizes = o; o = alignUp256(o + 4 * (size_t)n);
   p.total = o;
   return p;
-}
-
-int smCountD() {
-  // per device (a process may drive several); racing first calls write the same value
-  static int cached[64] = {};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
-  if (!cached[dev]) {
-    int v = 0;
-    cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
-    cached[dev] = v > 0 ? v : 148;
-  }
-  return cached[dev];
-}
-
-template <int KIND, int PB, int WARPS, bool STAGE, bool LUT64>
-int launchDecode(const DecodeScratch& sc, uint32_t m0, uint32_t m1, uint32_t part, uint64_t blockBound,
-                 cudaStream_t stream) {
-  auto kern = decodeKernel<KIND, PB, WARPS, STAGE, LUT64>;
-  const Options& opt = options();
-  // staging slot per warp: worst case for raw bytes; float kinds code exponent-like bytes that
-  // compress well, so a smaller slot (more resident warps) covers them and rare larger blocks
-  // take the direct-from-global path inside the kernel
-  uint32_t slotWords = 0;
-  if (STAGE) {
-    slotWords = opt.decode_slot_words > 0 ? (uint32_t)opt.decode_slot_words
-                                          : (KIND == kKindBytes ? maxBlockWords(PB) : 1536u);
-    slotWords = std::min(roundUp(slotWords, 8u), maxBlockWords(PB));
-  }
-  size_t smemBytes = (2 * kNumSymbols + 64) * 4 + ((WARPS + 1) & ~1) * 8 +
-                     (size_t)WARPS * kRingSlots * RowWriter<KIND>::kRingSlotBytes;
-  if (STAGE) smemBytes += (size_t)WARPS * (128u + slotWords * 2u);
-  // per instantiation and host thread; re-done when the thread's current device changes (function
-  // attributes are per device)
-  static thread_local int perSm = 0;
-  static thread_local size_t perSmKey = 0;
-  int devOrdinal = 0;
-  DGB_CUDA_TRY(cudaGetDevice(&devOrdinal));
-  const size_t occKey = smemBytes | ((size_t)(devOrdinal + 1) << 40);
-  if (perSm == 0 || perSmKey != occKey) {
-    DGB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-    int occ = 0;
-    DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, WARPS * 32, smemBytes));
-    perSm = std::max(occ, 1);
-    perSmKey = occKey;
-  }
-  // one resident wave; every warp gets the same number of blocks (rounds) when the batch is
-  // large, so no warp idles at the CTA barrier waiting for a neighbour's extra block
-  const uint64_t resident = (uint64_t)perSm * smCountD();
-  const uint64_t rounds = std::max<uint64_t>(1, (blockBound + resident * WARPS - 1) / (resident * WARPS));
-  const uint64_t want = (blockBound + WARPS * rounds - 1) / (WARPS * rounds);
-  const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(want, resident));
-  timerBegin(kSlotDecode, stream);
-  kern<<<grid, WARPS * 32, smemBytes, stream>>>(sc, m0, m1, part, slotWords);
-  DGB_CUDA_TRY(cudaGetLastError());
-  timerEnd(kSlotDecode, stream);
-  return DGB_OK;
-}
-
-// One variant is shipped per (kind, probBits): 8 warps per CTA, TMA-staged streams, 4-byte LUT
-// entries.  The alternatives measured in round 1 (4 warps, direct-from-global streams, 8-byte LUT
-// entries) were slower on every workload and are no longer instantiated.
-template <int KIND, int PB>
-int launchDecodeW(const DecodeScratch& sc, uint32_t m0, uint32_t m1, uint32_t part, uint64_t blockBound,
-                  cudaStream_t stream) {
-  return launchDecode<KIND, PB, 8, true, false>(sc, m0, m1, part, blockBound, stream);
 }
 
 // member table of the call in flight on this thread (decodeBatch fills it; count == 0: table in scratch)
@@ -861,7 +617,6 @@ template <int KIND, int PB, int WARPS>
 int launchDecodeFusedW(const DecodeScratch& sc, uint32_t n, uint64_t totalChunks,
                        uint32_t slotWordsOpt, uint8_t* outSuccess, uint32_t* outSize, bool checksum,
                        cudaStream_t stream) {
-  auto kern = decodeFusedKernel<KIND, PB, WARPS>;
   // staging slot per warp: worst case for raw bytes; float kinds code exponent-like bytes that
   // compress well, so a smaller slot (more resident warps) covers them and rare larger blocks
   // take the direct-from-global path inside the kernel
@@ -870,22 +625,13 @@ int launchDecodeFusedW(const DecodeScratch& sc, uint32_t n, uint64_t totalChunks
   const size_t smemBytes = (2 * kNumSymbols + 64) * 4 + ((WARPS + 1) & ~1) * 8 +
                            (size_t)WARPS * kRingSlots * RowWriter<KIND>::kRingSlotBytes +
                            (size_t)WARPS * (128u + slotWords * 2u);
-  static thread_local int perSm = 0;
-  static thread_local size_t perSmKey = 0;
-  int devOrdinal = 0;
-  DGB_CUDA_TRY(cudaGetDevice(&devOrdinal));
-  const size_t occKey = smemBytes | ((size_t)(devOrdinal + 1) << 40);
-  if (perSm == 0 || perSmKey != occKey) {
-    DGB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-    int occ = 0;
-    DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, WARPS * 32, smemBytes));
-    perSm = std::max(occ, 1);
-    perSmKey = occKey;
-  }
-  const uint64_t resident = (uint64_t)perSm * smCountD();
+  int perSm = 1;
+  const int rc = residentPerSm<decodeFusedKernel<KIND, PB, WARPS>>(WARPS * 32, smemBytes, 160 * 1024, &perSm);
+  if (rc != DGB_OK) return rc;
+  const uint64_t resident = (uint64_t)perSm * smCount();
   const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(resident, totalChunks));
   timerBegin(kSlotDecode, stream);
-  kern<<<grid, WARPS * 32, smemBytes, stream>>>(sc, decodeInline(), n, slotWords, outSuccess, outSize, checksum);
+  decodeFusedKernel<KIND, PB, WARPS><<<grid, WARPS * 32, smemBytes, stream>>>(sc, decodeInline(), n, slotWords, outSuccess, outSize, checksum);
   DGB_CUDA_TRY(cudaGetLastError());
   timerEnd(kSlotDecode, stream);
   return DGB_OK;
@@ -898,13 +644,12 @@ int launchDecodeFused(const DecodeScratch& sc, uint32_t n, uint64_t totalChunks,
   // warps per CTA = warps that share one LUT and meet at the barrier when a lease ends.  Float kinds: 8 (4 and
   // 10 / 20 measured: c3 146.5 / 142.1 / 151.2 us against 143.3).  Byte archives need the worst-case staging slot
   // (5.1 KiB per warp), which caps 8-warp CTAs at 32 resident warps per SM; 20-warp CTAs reach 40 (c2: 242 ->
-  // 233.5 us) -- used when the members are long enough to keep 20 warps busy through a lease.
+  // 233.5 us) -- used when the members are long enough to keep 20 warps busy through a lease.  Option values
+  // other than 20 (byte archives) select 8.
   int w = options().decode_warps;
   // (at 11 bits the LUT is 8 KiB and the slot 5.6 KiB per warp: a 20-warp CTA needs 126 KiB and fits once per
   // SM -- bench detail c2p11 fell from 884 to 800 GB/s -- so the wide CTA is used up to 10 bits only)
   if (w == 0) w = (KIND == kKindBytes && PB <= 10 && totalChunks * 8u >= 160ull * n) ? 20 : 8;
-  if (w == 4)
-    return launchDecodeFusedW<KIND, PB, 4>(sc, n, totalChunks, slotWordsOpt, outSuccess, outSize, checksum, stream);
   if constexpr (KIND == kKindBytes) {
     if (w == 20)
       return launchDecodeFusedW<KIND, PB, 20>(sc, n, totalChunks, slotWordsOpt, outSuccess, outSize, checksum, stream);
@@ -924,21 +669,6 @@ int decodeFusedKind(const DecodeScratch& sc, int pb, uint32_t n, uint64_t totalC
   }
 }
 
-template <int KIND>
-int decodeKind(const DecodeScratch& sc, int pb, bool checksum, uint32_t m0, uint32_t m1, uint32_t part,
-               uint64_t blockBound, uint8_t* outSuccess, uint32_t* outSize, cudaStream_t stream) {
-  timerBegin(kSlotPlan, stream);
-  planKernel<KIND><<<1, 1024, 0, stream>>>(sc, m0, m1, part, pb, outSuccess, outSize, checksum);
-  DGB_CUDA_TRY(cudaGetLastError());
-  timerEnd(kSlotPlan, stream);
-  switch (pb) {
-    case 9: return launchDecodeW<KIND, 9>(sc, m0, m1, part, blockBound, stream);
-    case 10: return launchDecodeW<KIND, 10>(sc, m0, m1, part, blockBound, stream);
-    case 11: return launchDecodeW<KIND, 11>(sc, m0, m1, part, blockBound, stream);
-    default: return DGB_ERR_INVALID_ARG;
-  }
-}
-
 }  // namespace
 
 size_t decodeTempBytes(int /*kind*/, uint32_t n) { return planDecodeScratch(n).total + 256; }
@@ -953,9 +683,7 @@ int decodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
   if (reinterpret_cast<uintptr_t>(temp) & 255u) return DGB_ERR_INVALID_ARG;
 
   const Options opt = options();  // one snapshot per call
-  const bool fused = opt.decode_fused != 0;
   static thread_local std::vector<MemberDesc> descStage;  // reused: no allocation on the steady-state path
-  static thread_local std::vector<uint64_t> weightStage;
   descStage.resize(n);
   MemberDesc* desc = descStage.data();
   const uint32_t wordBytes = kind == kKindF32 ? 4u : (kind == kKindBytes ? 1u : 2u);
@@ -968,9 +696,9 @@ int decodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
     desc[i].in = members[i].in;
     desc[i].out = members[i].out;
     desc[i].size = members[i].size;  // capacity
-    // single-launch path: block count bound from the capacity (>= 1: every header is visited once)
+    // block count bound from the capacity (>= 1: every header is visited once)
     const uint32_t blocks = std::max(1u, divUp(members[i].size, kBlockBytes));
-    desc[i].work0 = fused ? blocks : 0u;
+    desc[i].work0 = blocks;
     totalChunks += divUp(blocks, 8u);
   }
   uint8_t* base = static_cast<uint8_t*>(temp);
@@ -978,13 +706,12 @@ int decodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
   sc.members = reinterpret_cast<MemberDesc*>(base + dp.members);
   sc.next = reinterpret_cast<uint32_t*>(base + dp.next);
   sc.seen = sc.next + n;
-  sc.totals = reinterpret_cast<uint32_t*>(base + dp.totals);
   sc.checksum = reinterpret_cast<uint32_t*>(base + dp.checksum);
   sc.archiveChecksum = reinterpret_cast<uint32_t*>(base + dp.archiveChecksum);
   sc.sizes = reinterpret_cast<uint32_t*>(base + dp.sizes);
   // member table: inside the kernel parameters when it fits (the checksum pass reads it from scratch)
   InlineMembers& im = decodeInline();
-  const bool inlined = opt.inline_members != 0 && fused && !checksum && n <= kInlineMembers;
+  const bool inlined = opt.inline_members != 0 && !checksum && n <= kInlineMembers;
   im.count = inlined ? n : 0u;
   if (inlined) {
     std::memcpy(im.m, desc, sizeof(MemberDesc) * n);
@@ -993,75 +720,24 @@ int decodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
   }
   if (checksum) DGB_CUDA_TRY(cudaMemsetAsync(sc.checksum, 0, 4 * (size_t)n, stream));
 
-  if (fused) {
-    DGB_CUDA_TRY(cudaMemsetAsync(sc.next, 0, 8 * (size_t)n, stream));
-    const uint32_t slotOpt = opt.decode_slot_words > 0 ? (uint32_t)opt.decode_slot_words : 0u;
-    int rc;
-    switch (kind) {
-      case kKindBytes: rc = decodeFusedKind<kKindBytes>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
-      case kKindF16: rc = decodeFusedKind<kKindF16>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
-      case kKindBF16: rc = decodeFusedKind<kKindBF16>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
-      case kKindF32: rc = decodeFusedKind<kKindF32>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
-      default: return DGB_ERR_INVALID_ARG;
-    }
-    if (rc != DGB_OK) return rc;
-  } else {
-    // two-kernel path: sub-batches on internal streams: the plan kernel (pure latency) of one part
-    // hides behind the decode kernel of another, and the tail of one decode kernel overlaps the next
-    weightStage.resize(n);
-    uint64_t totalBytes = 0;
-    for (uint32_t i = 0; i < n; ++i) { weightStage[i] = (uint64_t)desc[i].size * wordBytes; totalBytes += weightStage[i]; }
-    const int parts = autoParts(kind, n, totalBytes, true);
-    uint32_t bounds[kMaxParts + 1];
-    splitParts(weightStage.data(), n, parts, bounds);
-    // joins the helper streams on every exit path (the caller reuses its scratch on return)
-    struct Join {
-      StreamPool* pool = nullptr;
-      cudaStream_t stream = nullptr;
-      bool forked[kMaxParts] = {};
-      ~Join() {
-        if (!pool) return;
-        for (int k = 0; k < kMaxParts; ++k)
-          if (forked[k] && cudaEventRecord(pool->done[k], pool->s[k]) == cudaSuccess) cudaStreamWaitEvent(stream, pool->done[k], 0);
-      }
-    } join;
-    StreamPool* pool = nullptr;
-    if (parts > 1) {
-      int prc = streamPool(&pool);
-      if (prc != DGB_OK) return prc;
-      DGB_CUDA_TRY(cudaEventRecord(pool->start, stream));
-      join.pool = pool;
-      join.stream = stream;
-    }
-    for (int part = 0; part < parts; ++part) {
-      const uint32_t m0 = bounds[part], m1 = bounds[part + 1];
-      if (m1 == m0) continue;
-      cudaStream_t ps = stream;
-      if (parts > 1) {
-        ps = pool->s[part];
-        DGB_CUDA_TRY(cudaStreamWaitEvent(ps, pool->start, 0));
-        join.forked[part] = true;
-      }
-      uint64_t partBound = 0;
-      for (uint32_t i = m0; i < m1; ++i) partBound += divUp(desc[i].size, kBlockBytes);
-      int rc;
-      switch (kind) {
-        case kKindBytes: rc = decodeKind<kKindBytes>(sc, pb, checksum, m0, m1, part, partBound, outSuccess_dev, outSize_dev, ps); break;
-        case kKindF16: rc = decodeKind<kKindF16>(sc, pb, checksum, m0, m1, part, partBound, outSuccess_dev, outSize_dev, ps); break;
-        case kKindBF16: rc = decodeKind<kKindBF16>(sc, pb, checksum, m0, m1, part, partBound, outSuccess_dev, outSize_dev, ps); break;
-        case kKindF32: rc = decodeKind<kKindF32>(sc, pb, checksum, m0, m1, part, partBound, outSuccess_dev, outSize_dev, ps); break;
-        default: return DGB_ERR_INVALID_ARG;
-      }
-      if (rc != DGB_OK) return rc;
-    }
-  }  // ~Join orders the helper streams before the caller's stream
+  DGB_CUDA_TRY(cudaMemsetAsync(sc.next, 0, 8 * (size_t)n, stream));
+  const uint32_t slotOpt = opt.decode_slot_words > 0 ? (uint32_t)opt.decode_slot_words : 0u;
+  int rc;
+  switch (kind) {
+    case kKindBytes: rc = decodeFusedKind<kKindBytes>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
+    case kKindF16: rc = decodeFusedKind<kKindF16>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
+    case kKindBF16: rc = decodeFusedKind<kKindBF16>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
+    case kKindF32: rc = decodeFusedKind<kKindF32>(sc, pb, n, totalChunks, slotOpt, outSuccess_dev, outSize_dev, checksum, stream); break;
+    default: return DGB_ERR_INVALID_ARG;
+  }
+  if (rc != DGB_OK) return rc;
 
   if (checksum) {
     // ans/GpuANSDecode.cuh:555-591 / float/GpuFloatDecompress.cuh:698-733: checksum the
     // output, compare with the archive's on the host (this path synchronises).
     // Float kinds: the checksum covers the first `size` BYTES (SURVEY A.6/B6); sc.sizes holds
     // the word count, which is exactly that byte count.
-    const int sms = smCountD();
+    const int sms = smCount();
     dim3 grid(n, std::max(1, std::min(64, 4 * sms / (int)std::max(1u, n))));
     checksumKernel<<<grid, 256, 0, stream>>>(sc);
     DGB_CUDA_TRY(cudaGetLastError());

@@ -23,7 +23,8 @@
 //                        blockWords[k].y).  Option encode_canonical selects encodeKernel:
 //                        ordered per-warp tickets + a decoupled look-back, block order,
 //                        byte-identical to the reference, slower.
-//   Large batches are cut by member into sub-batches on internal streams (capi.cu autoParts).
+//   Large float batches are cut by member into sub-batches on internal streams (capi.cu autoParts), so
+//   that K1 of one sub-batch (HBM-bound) runs beside K2 of the previous one (issue-bound).
 //
 // The archive produced is field-for-field the reference's (A.4 of SURVEY.md);
 // bits the reference leaves undefined are zero.
@@ -53,16 +54,6 @@ __device__ __forceinline__ uint4 ldStream16(const uint4* p) {
   return v;
 }
 
-// TMA landing buffer of a statistics item (fused launch): the item's whole slab arrives in shared
-// memory by one bulk copy (cp.async.bulk + mbarrier), so its HBM latency is covered by bytes in
-// flight, not by resident warps -- the item runs at full speed next to encoder CTAs.  The two-kernel
-// path (STAGED = false) keeps the register-pipelined global loads.
-struct StatsStage {
-  uint4* buf = nullptr;     // shared memory, 16 B aligned, >= slabVecs vectors
-  uint32_t bar = 0;         // shared address of the mbarrier
-  uint32_t* phase = nullptr;
-};
-
 struct EncodeScratch {
   MemberDesc* members;            // [n]
   uint32_t* hist;                 // [n][256]      (zeroed per call)
@@ -74,9 +65,6 @@ struct EncodeScratch {
   uint8_t* spill;                 // [resident warps][maxBlockWords] u16: overflow of small staging slots
   uint4* table;                   // [n][256] slots of 16 B (packed entries use the first half)
   bool wideTable;                 // entry format: EncEntryWide (16 B) or EncEntry (8 B)
-  // fused single-launch encoder only
-  const uint2* workIdx;           // [n + 1] {first stats item, first encode chunk} of member i
-  uint32_t* ready;                // [n]  (zeroed) 1 once the member's table is published
 };
 
 // ---------------------------------------------------------------------------
@@ -175,28 +163,25 @@ __device__ bool flushAndTicket(uint32_t (*sHist)[kNumSymbols], uint32_t* histGlo
 // K1 (bytes): histogram + checksum + normalisation epilogue.
 // grid = (n, Y): CTA (m, y) walks slabs y, y+Y, ... of member m.
 // ---------------------------------------------------------------------------
-// Slab accounting shared by host (work-item counts of the fused launch) and device.
-__host__ __device__ inline uint32_t bytesHeadLen(const void* in, uint32_t size) {
+__device__ inline uint32_t bytesHeadLen(const void* in, uint32_t size) {
   const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(in) & 15u);
   const uint32_t head = (16u - mis) & 15u;
   return size < head ? size : head;
 }
-__host__ __device__ inline uint32_t bytesSlabs(const void* in, uint32_t size, uint32_t slabVecs, bool doPass) {
+__device__ inline uint32_t bytesSlabs(const void* in, uint32_t size, uint32_t slabVecs, bool doPass) {
   if (!doPass) return 0u;
   const uint32_t nVec = (size - bytesHeadLen(in, size)) / 16u;
   const uint32_t s = divUp(nVec, slabVecs);
   return s > 0u ? s : (size > 0u ? 1u : 0u);
 }
 
-// Work of CTA y of Y on member m (Y = gridDim.y of the two-kernel path, the member's item count in
-// the fused kernel).  Returns true in the CTA that finished the member (its table is published).
-template <bool STAGED>
+// Work of CTA y of Y on member m.  Returns true in the CTA that finished the member (its table is
+// published).
 __device__ __forceinline__ bool statsBytesItem(const EncodeScratch& sc, uint32_t (*sHist)[kNumSymbols],
                                                const uint32_t* __restrict__ histogramGiven, int pb,
                                                bool useChecksum, uint32_t slabVecs, const MemberDesc& md,
                                                uint32_t m, uint32_t y,
-                                               uint32_t Y, uint32_t* __restrict__ outSize,
-                                               const StatsStage& stage = StatsStage()) {
+                                               uint32_t Y, uint32_t* __restrict__ outSize) {
   // shuffle => the histogram base is provably warp-uniform (ATOMS [R + UR], no per-symbol add)
   const uint32_t t = threadIdx.x, warp = __shfl_sync(0xffffffffu, t >> 5, 0);
   const uint8_t* in = static_cast<const uint8_t*>(md.in);
@@ -217,14 +202,6 @@ __device__ __forceinline__ bool statsBytesItem(const EncodeScratch& sc, uint32_t
   } else {
     if (y >= participants) return false;
     const uint4* vec = reinterpret_cast<const uint4*>(in + head);
-    if (STAGED && t == 0) {
-      const uint32_t v0 = y * slabVecs, v1 = min(nVec, v0 + slabVecs);
-      if (v1 > v0) {
-        fenceProxyAsync();  // the region was last touched through the generic proxy (coder staging)
-        mbarExpectTx(stage.bar, (v1 - v0) * 16u);
-        bulkLoad(smemAddr(stage.buf), vec + v0, (v1 - v0) * 16u, stage.bar);
-      }
-    }
 #pragma unroll
     for (int w = 0; w < kStatsWarps; ++w) sHist[w][t] = 0;
     __syncthreads();
@@ -236,16 +213,12 @@ __device__ __forceinline__ bool statsBytesItem(const EncodeScratch& sc, uint32_t
     }
     for (uint32_t slab = y; slab < nSlabs; slab += Y) {
       const uint32_t v0 = slab * slabVecs, v1 = min(nVec, v0 + slabVecs);
-      if (STAGED && v1 > v0) {  // one slab per item (Y == nSlabs): the copy was issued above
-        mbarWait(stage.bar, *stage.phase);
-        *stage.phase ^= 1u;
-      }
       for (uint32_t i0 = v0 + t; i0 < v1; i0 += kStatsUnroll * kStatsThreads) {
         uint4 vv[kStatsUnroll];
 #pragma unroll
         for (int k = 0; k < kStatsUnroll; ++k) {
           const uint32_t i = i0 + k * kStatsThreads;
-          vv[k] = i < v1 ? (STAGED ? stage.buf[i - v0] : ldStream16(vec + i)) : make_uint4(0, 0, 0, 0);
+          vv[k] = i < v1 ? ldStream16(vec + i) : make_uint4(0, 0, 0, 0);
         }
 #pragma unroll
         for (int k = 0; k < kStatsUnroll; ++k) {
@@ -285,7 +258,7 @@ statsBytesKernel(EncodeScratch sc, const __grid_constant__ InlineMembers im, con
                  bool useChecksum, uint32_t slabVecs, uint32_t memberBase, uint32_t* __restrict__ outSize) {
   __shared__ uint32_t sHist[kStatsWarps][kNumSymbols];
   const uint32_t m = blockIdx.x + memberBase;
-  statsBytesItem<false>(sc, sHist, histogramGiven, pb, useChecksum, slabVecs, memberAt(im, sc.members, m), m, blockIdx.y,
+  statsBytesItem(sc, sHist, histogramGiven, pb, useChecksum, slabVecs, memberAt(im, sc.members, m), m, blockIdx.y,
                         gridDim.y, outSize);
 }
 
@@ -311,12 +284,12 @@ __device__ __forceinline__ uint32_t rot16x2(uint32_t w) {
 }
 
 // member = [head elements up to the first 16 B boundary | 16 B vectors | tail elements]
-__host__ __device__ inline uint32_t floatHeadLen(const void* in, uint32_t size, uint32_t wordBytes) {
+__device__ inline uint32_t floatHeadLen(const void* in, uint32_t size, uint32_t wordBytes) {
   const uint32_t mis = (uint32_t)(reinterpret_cast<uintptr_t>(in) & 15u);
   const uint32_t head = ((16u - mis) & 15u) / wordBytes;
   return size < head ? size : head;
 }
-__host__ __device__ inline uint32_t floatSlabs(const void* in, uint32_t size, uint32_t wordBytes, uint32_t slabVecs) {
+__device__ inline uint32_t floatSlabs(const void* in, uint32_t size, uint32_t wordBytes, uint32_t slabVecs) {
   if (size == 0) return 0u;
   const uint32_t nVec = (size - floatHeadLen(in, size, wordBytes)) / (16u / wordBytes);
   const uint32_t s = divUp(nVec, slabVecs);
@@ -346,15 +319,15 @@ __device__ __forceinline__ uint32_t codedScalar(const uint8_t* in, uint32_t e) {
 
 // The vector body of a float statistics slab: vectors [v0, v1) of the member, 16 B each: a pure
 // read (the coder takes the coded byte out of the raw words itself and writes the stored planes).
-template <int FT, bool STAGED>
-__device__ __forceinline__ void histVectors(const uint4* __restrict__ vec, const StatsStage& stage, uint32_t v0,
-                                            uint32_t v1, uint32_t t, uint32_t* wh) {
+template <int FT>
+__device__ __forceinline__ void histVectors(const uint4* __restrict__ vec, uint32_t v0, uint32_t v1, uint32_t t,
+                                            uint32_t* wh) {
   for (uint32_t i0 = v0 + t; i0 < v1; i0 += kStatsUnroll * kStatsThreads) {
     uint4 vv[kStatsUnroll];
 #pragma unroll
     for (int k = 0; k < kStatsUnroll; ++k) {
       const uint32_t i = i0 + k * kStatsThreads;
-      vv[k] = i < v1 ? (STAGED ? stage.buf[i - v0] : ldStream16(vec + i)) : make_uint4(0, 0, 0, 0);
+      vv[k] = i < v1 ? ldStream16(vec + i) : make_uint4(0, 0, 0, 0);
     }
 #pragma unroll
     for (int k = 0; k < kStatsUnroll; ++k) {
@@ -371,12 +344,11 @@ __device__ __forceinline__ void histVectors(const uint4* __restrict__ vec, const
 }
 
 // Work of CTA y of Y on member m; returns true in the CTA that finished the member.
-template <int FT, bool STAGED>
+template <int FT>
 __device__ __forceinline__ bool statsFloatItem(const EncodeScratch& sc, uint32_t (*sHist)[kNumSymbols], int pb,
                                                bool useChecksum, uint32_t slabVecs, const MemberDesc& md,
                                                uint32_t m, uint32_t y,
-                                               uint32_t Y, uint32_t* __restrict__ outSize,
-                                               const StatsStage& stage = StatsStage()) {
+                                               uint32_t Y, uint32_t* __restrict__ outSize) {
   constexpr uint32_t EPV = (FT == DGB_FLOAT32) ? 4u : 8u;  // elements per 16 B vector
   constexpr uint32_t WB = (FT == DGB_FLOAT32) ? 4u : 2u;   // word bytes
   // shuffle => the histogram base is provably warp-uniform (ATOMS [R + UR], no per-symbol add)
@@ -398,14 +370,6 @@ __device__ __forceinline__ bool statsFloatItem(const EncodeScratch& sc, uint32_t
   } else {
     if (y >= participants) return false;
     const uint4* vec = reinterpret_cast<const uint4*>(in + (size_t)head * WB);
-    if (STAGED && t == 0) {
-      const uint32_t v0 = y * slabVecs, v1 = min(nVec, v0 + slabVecs);
-      if (v1 > v0) {
-        fenceProxyAsync();  // the region was last touched through the generic proxy (coder staging)
-        mbarExpectTx(stage.bar, (v1 - v0) * 16u);
-        bulkLoad(smemAddr(stage.buf), vec + v0, (v1 - v0) * 16u, stage.bar);
-      }
-    }
 #pragma unroll
     for (int w = 0; w < kStatsWarps; ++w) sHist[w][t] = 0;
     __syncthreads();
@@ -415,13 +379,9 @@ __device__ __forceinline__ bool statsFloatItem(const EncodeScratch& sc, uint32_t
     // ---- vector body ----
     for (uint32_t slab = y; slab < nSlabs; slab += Y) {
       const uint32_t v0 = slab * slabVecs, v1 = min(nVec, v0 + slabVecs);
-      if (STAGED && v1 > v0) {  // one slab per item (Y == nSlabs): the copy was issued above
-        mbarWait(stage.bar, *stage.phase);
-        *stage.phase ^= 1u;
-      }
       // four independent 16 B loads per thread are issued before any of them is consumed: the
       // kernel is a pure stream and was latency-bound with one load in flight
-      histVectors<FT, STAGED>(vec, stage, v0, v1, t, wh);
+      histVectors<FT>(vec, v0, v1, t, wh);
     }
     if (y == 0) {
       // ---- scalar head and tail (fewer than one vector each) ----
@@ -475,31 +435,8 @@ statsFloatKernel(EncodeScratch sc, const __grid_constant__ InlineMembers im, int
                  uint32_t memberBase, uint32_t* __restrict__ outSize) {
   __shared__ uint32_t sHist[kStatsWarps][kNumSymbols];
   const uint32_t m = blockIdx.x + memberBase;
-  statsFloatItem<FT, false>(sc, sHist, pb, useChecksum, slabVecs, memberAt(im, sc.members, m), m, blockIdx.y, gridDim.y,
+  statsFloatItem<FT>(sc, sHist, pb, useChecksum, slabVecs, memberAt(im, sc.members, m), m, blockIdx.y, gridDim.y,
                             outSize);
-}
-
-// K1 with the slab landed in shared memory by one TMA bulk copy per CTA (option stats_stage): the
-// bytes in flight per SM no longer depend on the number of resident statistics warps, so the kernel
-// keeps its bandwidth when it only gets the SM resources the coder of the previous sub-batch leaves
-// free.  gridDim.y must equal the slab count (one slab per CTA); dynamic shared memory = slab bytes.
-template <int FT>
-__global__ void __launch_bounds__(kStatsThreads)
-statsFloatStagedKernel(EncodeScratch sc, int pb, bool useChecksum, uint32_t slabVecs, uint32_t memberBase,
-                       uint32_t* __restrict__ outSize) {
-  extern __shared__ __align__(16) uint8_t stageSmem[];
-  __shared__ uint32_t sHist[kStatsWarps][kNumSymbols];
-  __shared__ __align__(8) unsigned long long sBar;
-  uint32_t phase = 0;
-  StatsStage stage;
-  stage.buf = reinterpret_cast<uint4*>(stageSmem);
-  stage.bar = smemAddr(&sBar);
-  stage.phase = &phase;
-  if (threadIdx.x == 0) mbarInit(stage.bar, 1);
-  fenceBarrierInit();
-  __syncthreads();
-  const uint32_t m = blockIdx.x + memberBase;
-  statsFloatItem<FT, true>(sc, sHist, pb, useChecksum, slabVecs, sc.members[m], m, blockIdx.y, gridDim.y, outSize, stage);
 }
 
 // ---------------------------------------------------------------------------
@@ -517,21 +454,6 @@ statsFloatStagedKernel(EncodeScratch sc, int pb, bool useChecksum, uint32_t slab
 #define DGB_ENC_GROUP_ROWS 16
 #endif
 constexpr int kEncGroupRows = DGB_ENC_GROUP_ROWS;  // rows per cp.async group
-
-__device__ __forceinline__ void cpAsync16(uint32_t dstSmem, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dstSmem), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cpAsyncCommit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cpAsyncWait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
-template <int OFF>
-__device__ __forceinline__ uint32_t ldsU8(uint32_t addr) {
-  uint32_t v;
-  asm volatile("ld.shared.u8 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(OFF));
-  return v;
-}
 
 // ---------------------------------------------------------------------------
 // Input side of the coder, per data kind.  The coder reads the member's RAW words (bytes, or the
@@ -871,12 +793,11 @@ __device__ __forceinline__ void spillOut(Spill& sp, uint32_t stageAddr, uint16_t
 // `stageAddr` (spilling to sp.area when the slot is small); float kinds also write the block's
 // stored plane(s).  Returns the TOTAL word count; the words not yet spilled are
 // stage[0 .. total - sp.spilled).
-template <bool WIDE, int KIND, bool TMA>
+template <bool WIDE, int KIND>
 __device__ __forceinline__ uint32_t encodeBlockWarp(const uint8_t* __restrict__ in, uint32_t n, uint32_t elem0,
                                                     const StoredPlanes& planes, uint32_t tabAddr, int pb,
                                                     uint32_t stageAddr, uint16_t* stage, Spill& sp,
-                                                    uint32_t ringAddr, uint32_t lane, uint32_t& stateOut,
-                                                    uint32_t ringBar = 0, uint32_t* ringPhase = nullptr) {
+                                                    uint32_t ringAddr, uint32_t lane, uint32_t& stateOut) {
   typedef EncIn<KIND> In;
   constexpr int U = kEncGroupRows;
   constexpr uint32_t WB = In::kWordBytes;
@@ -891,60 +812,32 @@ __device__ __forceinline__ uint32_t encodeBlockWarp(const uint8_t* __restrict__ 
   sp.spilled = 0;
   if ((reinterpret_cast<uintptr_t>(in) & 15u) == 0) {
     const uint32_t groups = fullRows / U;
-    if (TMA) {
-      // input rows arrive by TMA bulk copies (cp.async.bulk, one instruction of one lane per group of
-      // 16 rows) into a ring of slots, each with its own mbarrier, two groups ahead of the coder
-      auto issue = [&](uint32_t g, uint32_t slot) {
-        if (lane == 0) {
-          mbarExpectTx(ringBar + 8u * slot, kGroupBytes);
-          bulkLoad(ringAddr + slot * kGroupBytes, in + (size_t)g * kGroupBytes, kGroupBytes, ringBar + 8u * slot);
-        }
-      };
-      if (lane == 0) fenceProxyAsync();  // the ring was last touched through the generic proxy
-      if (groups > 0) issue(0, 0);
-      if (groups > 1) issue(1, 1);
-      uint32_t slot = 0, slotNext = 2 % In::kRingSlots, phases = *ringPhase;
-      for (uint32_t k = 0; k < groups; ++k) {
-        __syncwarp();  // every lane is done with the group that last sat in slotNext
-        if (k + 2 < groups) issue(k + 2, slotNext);
-        if (sp.area && wa - stageAddr > sp.limitBytes) spillOut(sp, stageAddr, stage, wa, lane);
-        mbarWait(ringBar + 8u * slot, (phases >> slot) & 1u);
-        phases ^= 1u << slot;
-        const uint32_t slotAddr = ringAddr + slot * kGroupBytes;
-        if (KIND != kKindBytes) In::storeGroup(slotAddr, planes, elem0 + k * (U * 32), lane);
-        encodeGroup<WIDE, KIND>(state, slotAddr + lane * WB, rc, wa);
-        slot = slot + 1 == In::kRingSlots ? 0u : slot + 1;
-        slotNext = slotNext + 1 == In::kRingSlots ? 0u : slotNext + 1;
-      }
-      *ringPhase = phases;
-    } else {
-      // input rows stream through the cp.async ring, two groups ahead of the encoder
-      const uint8_t* src = in + lane * 16u;
-      const uint32_t dst = ringAddr + lane * 16u;
-      auto issue = [&](uint32_t g, uint32_t slot) {
+    // input rows stream through the cp.async ring, two groups ahead of the encoder
+    const uint8_t* src = in + lane * 16u;
+    const uint32_t dst = ringAddr + lane * 16u;
+    auto issue = [&](uint32_t g, uint32_t slot) {
 #pragma unroll
-        for (uint32_t c = 0; c < kChunks; ++c)
-          cpAsync16(dst + slot * kGroupBytes + c * 512u, src + (size_t)g * kGroupBytes + c * 512u);
-      };
-      if (groups > 0) issue(0, 0);
+      for (uint32_t c = 0; c < kChunks; ++c)
+        cpAsync16(dst + slot * kGroupBytes + c * 512u, src + (size_t)g * kGroupBytes + c * 512u);
+    };
+    if (groups > 0) issue(0, 0);
+    cpAsyncCommit();
+    if (groups > 1) issue(1, 1);
+    cpAsyncCommit();
+    uint32_t slot = 0, slotNext = 2 % In::kRingSlots;
+    for (uint32_t k = 0; k < groups; ++k) {
+      if (sp.area && wa - stageAddr > sp.limitBytes) spillOut(sp, stageAddr, stage, wa, lane);
+      cpAsyncWait<1>();  // group k has landed (group k + 1 may still be in flight)
+      // one warp barrier does both jobs: every lane sees group k, and every lane is done reading group
+      // k - 1, whose ring slot (three-slot ring) the request below overwrites
+      __syncwarp();
+      if (k + 2 < groups) issue(k + 2, slotNext);
       cpAsyncCommit();
-      if (groups > 1) issue(1, 1);
-      cpAsyncCommit();
-      uint32_t slot = 0, slotNext = 2 % In::kRingSlots;
-      for (uint32_t k = 0; k < groups; ++k) {
-        if (sp.area && wa - stageAddr > sp.limitBytes) spillOut(sp, stageAddr, stage, wa, lane);
-        cpAsyncWait<1>();  // group k has landed (group k + 1 may still be in flight)
-        // one warp barrier does both jobs: every lane sees group k, and every lane is done reading group
-        // k - 1, whose ring slot (three-slot ring) the request below overwrites
-        __syncwarp();
-        if (k + 2 < groups) issue(k + 2, slotNext);
-        cpAsyncCommit();
-        const uint32_t slotAddr = ringAddr + slot * kGroupBytes;
-        if (KIND != kKindBytes) In::storeGroup(slotAddr, planes, elem0 + k * (U * 32), lane);
-        encodeGroup<WIDE, KIND>(state, slotAddr + lane * WB, rc, wa);
-        slot = slot + 1 == In::kRingSlots ? 0u : slot + 1;
-        slotNext = slotNext + 1 == In::kRingSlots ? 0u : slotNext + 1;
-      }
+      const uint32_t slotAddr = ringAddr + slot * kGroupBytes;
+      if (KIND != kKindBytes) In::storeGroup(slotAddr, planes, elem0 + k * (U * 32), lane);
+      encodeGroup<WIDE, KIND>(state, slotAddr + lane * WB, rc, wa);
+      slot = slot + 1 == In::kRingSlots ? 0u : slot + 1;
+      slotNext = slotNext + 1 == In::kRingSlots ? 0u : slotNext + 1;
     }
     r = groups * U;
   }
@@ -1086,8 +979,8 @@ __global__ void encodeKernel(EncodeScratch sc, int pb, bool useChecksum,
     const uint32_t blockLen = min(kBlockBytes, size - start);
     uint32_t state;
     Spill sp{nullptr, 0u, 0u};  // worst-case sized slot: never spills
-    const uint32_t words = encodeBlockWarp<false, KIND, false>(ansIn + (size_t)start * EncIn<KIND>::kWordBytes, blockLen, start, planes,
-                                                               tabAddr, pb, stageAddr, myStage, sp, ringAddr, lane, state);
+    const uint32_t words = encodeBlockWarp<false, KIND>(ansIn + (size_t)start * EncIn<KIND>::kWordBytes, blockLen, start, planes,
+                                                        tabAddr, pb, stageAddr, myStage, sp, ringAddr, lane, state);
     const uint32_t padded = roundUp(words, 8u);
 
     // ---- packed offset of this block: look-back over the member's earlier tickets ----
@@ -1142,25 +1035,17 @@ __host__ __device__ constexpr uint32_t encFastWarpSmem(uint32_t slotWords, int k
   return encRingBytes(kind) + slotWords * 2u;  // ring + staging
 }
 
-// Per-warp view of the CTA's dynamic shared memory: [input ring | staging slot] per warp.
-#ifndef DGB_ENC_TMA
-#define DGB_ENC_TMA 0
-#endif
-// input rows by per-lane cp.async (0, default) or by TMA bulk copy (1).  A/B on B200, encode call, cp.async / TMA:
-// c3 185.7 / 192.1 us, c4 209.5 / 212.0, c2 358.0 / 363.3 (profiles/r02_ab_tma_input_ring.txt): one lane issuing the bulk
-// copy and 32 lanes polling the mbarrier cost more than the two LDGSTS per lane they replace.
-constexpr bool kEncTma = DGB_ENC_TMA != 0;
-
+// Per-warp view of the CTA's dynamic shared memory: [input ring | staging slot] per warp.  Input rows
+// arrive by per-lane cp.async: a TMA bulk copy per group (one lane issuing, 32 lanes polling an
+// mbarrier) measured slower on B200, encode call c3 185.7 vs 192.1 us, c4 209.5 vs 212.0, c2 358.0 vs
+// 363.3 (profiles/r02_ab_tma_input_ring.txt).
 struct WarpSmem {
   uint32_t ringAddr, stageAddr;
   uint16_t* stage;
   Spill sp;
-  uint32_t ringBar;    // shared address of this warp's ring mbarriers (one per slot)
-  uint32_t ringPhase;  // bit s = parity the next wait on slot s expects
 };
 __device__ __forceinline__ WarpSmem warpSmem(const EncodeScratch& sc, uint8_t* smem, uint32_t warp, uint32_t W,
-                                             uint32_t slotWords, int pb, int kind, uint32_t spillWarpBase,
-                                             unsigned long long (*ringBars)[4]) {
+                                             uint32_t slotWords, int pb, int kind, uint32_t spillWarpBase) {
   WarpSmem ws;
   uint8_t* mine = smem + (size_t)warp * encFastWarpSmem(slotWords, kind);
   ws.ringAddr = smemAddr(mine);
@@ -1171,11 +1056,6 @@ __device__ __forceinline__ WarpSmem warpSmem(const EncodeScratch& sc, uint8_t* s
   ws.sp.spilled = 0;
   ws.stage = reinterpret_cast<uint16_t*>(mine + encRingBytes(kind));
   ws.stageAddr = smemAddr(ws.stage);
-  ws.ringBar = smemAddr(&ringBars[warp][0]);  // static shared memory: the dynamic region is reused by statistics items
-  ws.ringPhase = 0;
-  if (kEncTma && (threadIdx.x & 31u) == 0) {
-    for (uint32_t k = 0; k < 4; ++k) mbarInit(ws.ringBar + 8u * k, 1);
-  }
   return ws;
 }
 
@@ -1223,9 +1103,9 @@ __device__ __forceinline__ void encodeMemberBlocks(const EncodeScratch& sc, cons
     const uint32_t start = block * kBlockBytes;
     const uint32_t blockLen = min(kBlockBytes, size - start);
     uint32_t state;
-    const uint32_t words = encodeBlockWarp<WIDE, KIND, kEncTma>(ansIn + (size_t)start * EncIn<KIND>::kWordBytes, blockLen, start,
-                                                                planes, tabAddr, pb, ws.stageAddr, ws.stage, ws.sp, ws.ringAddr,
-                                                                lane, state, ws.ringBar, &ws.ringPhase);
+    const uint32_t words = encodeBlockWarp<WIDE, KIND>(ansIn + (size_t)start * EncIn<KIND>::kWordBytes, blockLen, start,
+                                                       planes, tabAddr, pb, ws.stageAddr, ws.stage, ws.sp, ws.ringAddr,
+                                                       lane, state);
     const uint32_t padded = roundUp(words, 8u);
     // take a place in the data section: one 64-bit atomic hands out the word offset (low half)
     // and counts finished blocks (high half), so no fence is needed to order the two
@@ -1264,12 +1144,7 @@ encodeKernelFast(EncodeScratch sc, const __grid_constant__ InlineMembers im, int
   const uint32_t t = threadIdx.x, lane = t & 31u;
   const uint32_t warp = __shfl_sync(0xffffffffu, t >> 5, 0);
   const uint32_t W = blockDim.x >> 5;
-  __shared__ __align__(8) unsigned long long sRingBar[8][4];
-  WarpSmem ws = warpSmem(sc, smem, warp, W, slotWords, pb, KIND, spillWarpBase, sRingBar);
-  if (kEncTma) {
-    fenceBarrierInit();
-    __syncthreads();
-  }
+  WarpSmem ws = warpSmem(sc, smem, warp, W, slotWords, pb, KIND, spillWarpBase);
   const uint32_t tabAddr = smemAddr(sTab);
 
   const uint64_t g = gridDim.x, span = blockEnd - blockBegin;
@@ -1299,191 +1174,34 @@ encodeKernelFast(EncodeScratch sc, const __grid_constant__ InlineMembers im, int
   }
 }
 
-// ---------------------------------------------------------------------------
-// Fused single-launch encoder (option encode_fused=1; measured no faster than the two-kernel path, DESIGN.md
-// section 4, so not the default).  One persistent grid; every CTA picks, at each step, one
-// of two kinds of work from two global counters:
-//   * a STATISTICS item  = one slab of one member (the body of K1 above: histogram (+ split, +
-//     checksum); the CTA that finishes a member normalises, publishes pdf + table and sets the
-//     member's `ready` flag), or
-//   * an ENCODE chunk    = a run of 4 KiB blocks of one member (the body of K2), which needs the
-//     member's flag.
-// Chunks are claimed in member order, and a CTA whose chunk is not ready yet works on statistics
-// items (which have no dependencies) instead of waiting, so the HBM-latency-bound statistics pass
-// and the issue-bound coder share every SM and balance themselves; one CTA in `statsEvery` prefers
-// statistics so that the tables stay ahead of the coders.  Progress never depends on co-residency:
-// a claimed item is always held by a running CTA, and the only wait (chunk claimed, member not
-// ready, no statistics left to claim) is for items other running CTAs hold.
-// The reference runs 7-10 kernels for this (SURVEY.md 3.1); its README lists a single cooperative
-// kernel as a next step (README.md:103).
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t ldAcquire(const uint32_t* p) {
-  uint32_t v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void stRelease(uint32_t* p, uint32_t v) {
-  asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-enum FusedAct : uint32_t { kActExit = 0, kActWait = 1, kActStats = 2, kActEncode = 3 };
-constexpr uint32_t kNoChunk = 0xffffffffu;
-
-template <int KIND, bool WIDE, bool STAGED>
-__global__ void __launch_bounds__(kStatsThreads, 4)
-encodeFusedKernel(EncodeScratch sc, const uint32_t* __restrict__ histogramGiven, int pb, bool useChecksum,
-                  uint32_t numMembers, uint32_t totalItems, uint32_t totalChunks, uint32_t slabVecs,
-                  uint32_t chunkBlocks, uint32_t slotWords, uint32_t statsEvery,
-                  uint32_t* __restrict__ outSize) {
-  // dynamic shared memory: per-warp [ring | staging slot] while encoding, the per-warp histograms
-  // while a statistics item runs (never both: the roles alternate between CTA-wide barriers)
-  extern __shared__ __align__(16) uint8_t smem[];
-  __shared__ __align__(16) uint4 sTab[WIDE ? kNumSymbols : kNumSymbols / 2];
-  __shared__ uint32_t sCtl[8];
-  __shared__ __align__(8) unsigned long long sStageBar;
-  uint32_t (*sHist)[kNumSymbols] = reinterpret_cast<uint32_t (*)[kNumSymbols]>(smem);
-  const uint32_t t = threadIdx.x, lane = t & 31u;
-  const uint32_t warp = __shfl_sync(0xffffffffu, t >> 5, 0);
-  constexpr uint32_t W = kStatsThreads / 32;
-  // statistics items: histograms in the first 8 KiB of the dynamic region, the slab's landing
-  // buffer in the rest (the host sizes slabVecs to fit)
-  uint32_t stagePhase = 0;
-  StatsStage stage;
-  stage.buf = reinterpret_cast<uint4*>(smem + sizeof(uint32_t) * kStatsWarps * kNumSymbols);
-  stage.bar = smemAddr(&sStageBar);
-  stage.phase = &stagePhase;
-  if (STAGED) {
-    if (t == 0) mbarInit(stage.bar, 1);
-    fenceBarrierInit();
-    __syncthreads();
-  }
-  __shared__ __align__(8) unsigned long long sRingBar[8][4];
-  WarpSmem ws = warpSmem(sc, smem, warp, W, slotWords, pb, KIND, 0u, sRingBar);
-  if (kEncTma) {
-    fenceBarrierInit();
-    __syncthreads();
-  }
-  const uint32_t tabAddr = smemAddr(sTab);
-  const bool preferStats = statsEvery != 0u && (blockIdx.x % statsEvery) == 0u;
-
-  // claim state (meaningful in thread 0; the decision is broadcast through sCtl)
-  uint32_t chunk = kNoChunk, chunkMember = 0, itemMember = 0;
-  bool chunksLeft = totalChunks != 0u, statsLeft = totalItems != 0u;
-  uint32_t tabMember = 0xffffffffu;
-
-  for (;;) {
-    if (t == 0) {
-      uint32_t act = kActWait, arg = 0, m = 0;
-      uint32_t item = 0xffffffffu;
-      if (preferStats && statsLeft) {
-        item = atomicAdd(sc.ticket + 0, 1u);
-        if (item >= totalItems) { statsLeft = false; item = 0xffffffffu; }
-      }
-      if (item == 0xffffffffu) {
-        if (chunk == kNoChunk && chunksLeft) {
-          chunk = atomicAdd(sc.ticket + 1, 1u);
-          if (chunk >= totalChunks) { chunk = kNoChunk; chunksLeft = false; }
-        }
-        if (chunk != kNoChunk) {
-          while (__ldg(&sc.workIdx[chunkMember + 1].y) <= chunk) ++chunkMember;  // claims only grow
-          if (ldAcquire(sc.ready + chunkMember) != 0u) { act = kActEncode; arg = chunk; m = chunkMember; chunk = kNoChunk; }
-        }
-        if (act == kActWait && statsLeft) {
-          item = atomicAdd(sc.ticket + 0, 1u);
-          if (item >= totalItems) { statsLeft = false; item = 0xffffffffu; }
-        }
-        if (act == kActWait && item == 0xffffffffu && chunk == kNoChunk) act = kActExit;  // nothing left anywhere
-      }
-      if (item != 0xffffffffu) {
-        while (__ldg(&sc.workIdx[itemMember + 1].x) <= item) ++itemMember;
-        act = kActStats; arg = item; m = itemMember;
-      }
-      sCtl[0] = act; sCtl[1] = arg; sCtl[2] = m;
-    }
-    __syncthreads();
-    const uint32_t act = sCtl[0], arg = sCtl[1], m = sCtl[2];
-    if (act == kActExit) break;
-    if (act == kActStats) {
-      const uint2 w0 = __ldg(&sc.workIdx[m]), w1 = __ldg(&sc.workIdx[m + 1]);
-      bool finished;
-      if (KIND == kKindBytes) {
-        finished = statsBytesItem<STAGED>(sc, sHist, histogramGiven, pb, useChecksum, slabVecs, sc.members[m], m, arg - w0.x,
-                                          w1.x - w0.x, outSize, stage);
-      } else {
-        finished = statsFloatItem<KIND == kKindBytes ? DGB_FLOAT16 : KIND, STAGED>(
-            sc, sHist, pb, useChecksum, slabVecs, sc.members[m], m, arg - w0.x, w1.x - w0.x, outSize, stage);
-      }
-      if (finished) {
-        // table, pdf and (through the ticket chain) every comp / stored byte of the member are
-        // visible before the flag
-        __threadfence();
-        __syncthreads();
-        if (t == 0) stRelease(sc.ready + m, 1u);
-      }
-    } else if (act == kActEncode) {
-      const MemberDesc md = sc.members[m];
-      if (tabMember != m) {
-        loadTable<WIDE>(sc, sTab, m);
-        tabMember = m;
-        __syncthreads();
-      }
-      const uint32_t nb = divUp(md.size, kBlockBytes);
-      const uint32_t first = (arg - __ldg(&sc.workIdx[m].y)) * chunkBlocks;
-      encodeMemberBlocks<WIDE, KIND>(sc, md, m, first, min(nb, first + chunkBlocks), pb, useChecksum, tabAddr, ws,
-                                     warp, W, lane, outSize);
-    } else {
-      __nanosleep(256);
-    }
-    __syncthreads();  // sCtl, the table slot and the dynamic region are reused by the next step
-  }
-}
-
-size_t alignUp256(size_t v) { return (v + 255) & ~size_t(255); }
-
-int smCount() {
-  // per device (a process may drive several); racing first calls write the same value
-  static int cached[64] = {};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return 148;
-  if (!cached[dev]) {
-    int v = 0;
-    cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev);
-    cached[dev] = v > 0 ? v : 148;
-  }
-  return cached[dev];
-}
-
 struct ScratchPlan {
-  size_t members, workIdx, uploadEnd, zeroBegin, hist, histDone, checksum, ticket, allocDone, ready, zeroEnd, lookback,
-      lookbackEnd, table, spill, total;
+  size_t members, zeroBegin, hist, histDone, checksum, ticket, allocDone, zeroEnd, lookback, lookbackEnd, table, spill,
+      total;
   uint32_t spillWarps;
 };
 
 // Encoder warps that may need a spill slot (one slot = the worst-case stream of one block): never
 // more than the device can hold resident (64 warps per SM), never more than the batch has work
 // for, so small batches get small scratch (the reference's scratch scales with the batch too).
+// The bound also caps the coder grid (spillWarpsPerPart / W in encodeBatch), so it is part of the
+// launch configuration, not only of the scratch size.
 uint32_t spillWarpBound(uint32_t n, uint64_t totalBlocks) {
   const uint64_t resident = 64ull * (uint64_t)smCount();
-  const uint64_t work = 8ull * ((uint64_t)n * 2ull + totalBlocks);  // 8 warps per CTA, <= items + chunks CTAs
+  // up to 8 warps per CTA; a coder grid has at most one CTA per block, plus a slack of two CTAs per member
+  const uint64_t work = 8ull * ((uint64_t)n * 2ull + totalBlocks);
   return (uint32_t)std::min(resident, work);
 }
 
 ScratchPlan planScratch(int kind, uint32_t n, uint32_t maxSize, uint32_t totalTickets, uint32_t spillWarps) {
   ScratchPlan p{};
   size_t o = 0;
-  // uploaded in one copy: member descriptors, then the fused launch's work index
-  p.members = o; o += sizeof(MemberDesc) * (size_t)n;
-  o = (o + 15) & ~size_t(15);
-  p.workIdx = o; o += sizeof(uint2) * ((size_t)n + 1);
-  p.uploadEnd = o;
-  o = alignUp256(o);
+  p.members = o; o = alignUp256(o + sizeof(MemberDesc) * (size_t)n);  // uploaded unless the kernel parameters carry it
   p.zeroBegin = o;
   p.hist = o; o = alignUp256(o + sizeof(uint32_t) * kNumSymbols * (size_t)n);
   p.histDone = o; o = alignUp256(o + sizeof(uint32_t) * (size_t)n);
   p.checksum = o; o = alignUp256(o + sizeof(uint32_t) * (size_t)n);
   p.ticket = o; o = alignUp256(o + 16);
   p.allocDone = o; o = alignUp256(o + sizeof(unsigned long long) * (size_t)n);
-  p.ready = o; o = alignUp256(o + sizeof(uint32_t) * (size_t)n);
   p.zeroEnd = o;
   // look-back descriptors: canonical (ordered) layout only; cleared only then
   p.lookback = o; o = alignUp256(o + sizeof(unsigned long long) * (size_t)totalTickets);
@@ -1515,7 +1233,7 @@ struct ForkGuard {
 
 // per-thread reusable host staging (no allocation on the steady-state call path)
 struct HostStage {
-  std::vector<uint8_t> upload;
+  std::vector<MemberDesc> desc;
   std::vector<uint64_t> weight;
 };
 HostStage& hostStage() {
@@ -1523,66 +1241,15 @@ HostStage& hostStage() {
   return h;
 }
 
-template <int KIND, bool WIDE, bool STAGED>
-int launchFused(const EncodeScratch& sc, const uint32_t* histogram_dev, int pb, bool checksum, uint32_t n,
-                uint32_t totalItems, uint32_t totalChunks, uint32_t slabVecs, uint32_t chunkBlocks,
-                uint32_t slotWords, uint32_t statsEvery, uint32_t spillWarps, uint32_t* outSize_dev,
-                cudaStream_t stream) {
-  auto kern = encodeFusedKernel<KIND, WIDE, STAGED>;
-  constexpr uint32_t W = kStatsThreads / 32;
-  const size_t smemBytes = (size_t)W * encFastWarpSmem(slotWords, KIND);
-  static thread_local int perSm = 0;
-  static thread_local size_t perSmKey = 0;
-  int devOrdinal = 0;
-  DGB_CUDA_TRY(cudaGetDevice(&devOrdinal));
-  const size_t occKey = smemBytes | ((size_t)(devOrdinal + 1) << 40);
-  if (perSm == 0 || perSmKey != occKey) {
-    DGB_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-    int occ = 0;
-    DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, (int)kStatsThreads, smemBytes));
-    perSm = std::max(occ, 1);
-    perSmKey = occKey;
-  }
-  uint64_t grid = (uint64_t)perSm * (uint64_t)smCount();
-  grid = std::min<uint64_t>(grid, (uint64_t)totalItems + totalChunks);
-  grid = std::min<uint64_t>(grid, spillWarps / W);  // every warp owns a spill slot
-  grid = std::max<uint64_t>(grid, 1);
-  timerBegin(kSlotFused, stream);
-  kern<<<(uint32_t)grid, kStatsThreads, smemBytes, stream>>>(sc, histogram_dev, pb, checksum, n, totalItems, totalChunks,
-                                                             slabVecs, chunkBlocks, slotWords, statsEvery, outSize_dev);
-  DGB_CUDA_TRY(cudaGetLastError());
-  timerEnd(kSlotFused, stream);
-  return DGB_OK;
-}
-
-// K2 of the two-kernel path for one data kind: variant 0 = canonical (ordered, packed table),
-// 1 = fast + packed table, 2 = fast + wide table.  Launch attributes and occupancy are cached per
-// host thread and (variant, shared-memory size, device).
+// K2 for one data kind: variant 0 = canonical (ordered, packed table), 1 = fast + packed table,
+// 2 = fast + wide table.
 template <int KIND>
 struct K2Launcher {
   static int residentPerSm(int variant, uint32_t W, size_t smemBytes, int* out) {
-    static thread_local size_t keySmem = 0;
-    static thread_local uint32_t keyW = 0;
-    static thread_local int keyVariant = -1, keyDev = -1, perSm = 1;
-    int dev = 0;
-    DGB_CUDA_TRY(cudaGetDevice(&dev));
-    if (keySmem != smemBytes || keyW != W || keyVariant != variant || keyDev != dev) {
-      int occ = 0;
-      if (variant == 0) {
-        DGB_CUDA_TRY(cudaFuncSetAttribute(encodeKernel<KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-        DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, encodeKernel<KIND>, (int)(W * 32), smemBytes));
-      } else if (variant == 1) {
-        DGB_CUDA_TRY(cudaFuncSetAttribute(encodeKernelFast<false, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-        DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, encodeKernelFast<false, KIND>, (int)(W * 32), smemBytes));
-      } else {
-        DGB_CUDA_TRY(cudaFuncSetAttribute(encodeKernelFast<true, KIND>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(200 * 1024)));
-        DGB_CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, encodeKernelFast<true, KIND>, (int)(W * 32), smemBytes));
-      }
-      perSm = std::max(occ, 1);
-      keySmem = smemBytes; keyW = W; keyVariant = variant; keyDev = dev;
-    }
-    *out = perSm;
-    return DGB_OK;
+    const int threads = (int)(W * 32), maxSmem = 200 * 1024;
+    if (variant == 0) return dgb::residentPerSm<encodeKernel<KIND>>(threads, smemBytes, maxSmem, out);
+    if (variant == 1) return dgb::residentPerSm<encodeKernelFast<false, KIND>>(threads, smemBytes, maxSmem, out);
+    return dgb::residentPerSm<encodeKernelFast<true, KIND>>(threads, smemBytes, maxSmem, out);
   }
   static void launch(int variant, uint32_t grid, uint32_t W, size_t smemBytes, cudaStream_t ps, const EncodeScratch& sc,
                      const InlineMembers& im, int pb, bool checksum, uint32_t n, uint32_t totalTickets, uint32_t blockBegin, uint32_t blockEnd,
@@ -1621,35 +1288,22 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
   if (pb < 9 || pb > 11) return DGB_ERR_INVALID_ARG;
   if (kind != kKindBytes && histogram_dev) return DGB_ERR_INVALID_ARG;
   const Options opt = options();  // one snapshot per call
-  const uint32_t W = (uint32_t)std::max(1, std::min(opt.encode_warps, 8));  // warps per CTA (two-kernel path)
+  const uint32_t W = (uint32_t)std::max(1, std::min(opt.encode_warps, 8));  // warps per coder CTA
   const uint32_t elemBytes = kind == kKindF32 ? 4u : (kind == kKindBytes ? 1u : 2u);
   const bool canonical = opt.encode_canonical != 0;
-  const bool fused = !canonical && opt.encode_fused != 0;
-  // staging slot of the fast / fused encoder (spills to global scratch when a block needs more)
+  // staging slot of the fast encoder (spills to global scratch when a block needs more)
   uint32_t slotWords = opt.encode_slot_words > 0 ? (uint32_t)opt.encode_slot_words
                                                  : (kind == kKindBytes ? 2304u : 1536u);
   slotWords = std::max<uint32_t>(roundUp(slotWords, 8u), kEncGroupRows * 32u + 264u);
   slotWords = std::min(slotWords, maxBlockWords(pb));
-  // statistics slab: the two-kernel path streams it through registers; the fused launch lands it in
-  // the part of the CTA's dynamic shared memory that the histograms do not use (TMA bulk copy)
-  const bool staged = fused && opt.fused_stage != 0;
-  uint32_t slabVecs = (uint32_t)std::max(1, opt.hist_slab_kb) * 1024u / 16u;
-  if (staged) {
-    const uint32_t stageBytes = (kStatsThreads / 32) * encFastWarpSmem(slotWords, kind) - (uint32_t)sizeof(uint32_t) * kStatsWarps * kNumSymbols;
-    slabVecs = std::max(1u, std::min(slabVecs, stageBytes / 16u));
-  }
-  const uint32_t chunkBlocks = (uint32_t)std::max(1, std::min(opt.fused_chunk_blocks, 4096));
-  const bool doPass = histogram_dev == nullptr || checksum;
+  const uint32_t slabVecs = (uint32_t)std::max(1, opt.hist_slab_kb) * 1024u / 16u;  // statistics slab
 
-  // ---- member table + work index (host staging, one upload) ----
+  // ---- member table (host staging) ----
   HostStage& hs = hostStage();
-  const size_t descBytes = sizeof(MemberDesc) * (size_t)n;
-  const size_t idxOff = (descBytes + 15) & ~size_t(15);
-  hs.upload.resize(idxOff + sizeof(uint2) * ((size_t)n + 1));
-  MemberDesc* desc = reinterpret_cast<MemberDesc*>(hs.upload.data());
-  uint2* workIdx = reinterpret_cast<uint2*>(hs.upload.data() + idxOff);
+  hs.desc.resize(n);
+  MemberDesc* desc = hs.desc.data();
   uint32_t maxSize = 0;
-  uint64_t tickets = 0, items = 0, chunks = 0;
+  uint64_t tickets = 0;
   for (uint32_t i = 0; i < n; ++i) {
     const HostMember& hm = members[i];
     if ((hm.size && !hm.in) || !hm.out) return DGB_ERR_INVALID_ARG;
@@ -1663,17 +1317,10 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
     desc[i].out = hm.out;
     desc[i].size = hm.size;
     desc[i].work0 = (uint32_t)tickets;
-    workIdx[i] = make_uint2((uint32_t)items, (uint32_t)chunks);
-    const uint32_t nb = ticketsFor(hm.size);
-    tickets += nb;
-    chunks += divUp(nb, chunkBlocks);
-    const uint32_t slabs = kind == kKindBytes ? bytesSlabs(hm.in, hm.size, slabVecs, doPass)
-                                              : floatSlabs(hm.in, hm.size, elemBytes, slabVecs);
-    items += std::max(1u, slabs);
+    tickets += ticketsFor(hm.size);
     maxSize = std::max(maxSize, hm.size);
-    if (tickets > 0x7fffffffull || items > 0x7fffffffull) return DGB_ERR_TOO_LARGE;
+    if (tickets > 0x7fffffffull) return DGB_ERR_TOO_LARGE;
   }
-  workIdx[n] = make_uint2((uint32_t)items, (uint32_t)chunks);
   const uint32_t totalTickets = (uint32_t)tickets;
   const ScratchPlan sp = planScratch(kind, n, maxSize, totalTickets, spillWarpBound(n, tickets));
   if (!temp || tempBytes < sp.total || (reinterpret_cast<uintptr_t>(temp) & 255u))
@@ -1682,26 +1329,23 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
   uint8_t* base = static_cast<uint8_t*>(temp);
   EncodeScratch sc;
   sc.members = reinterpret_cast<MemberDesc*>(base + sp.members);
-  sc.workIdx = reinterpret_cast<const uint2*>(base + sp.workIdx);
   sc.hist = reinterpret_cast<uint32_t*>(base + sp.hist);
   sc.histDone = reinterpret_cast<uint32_t*>(base + sp.histDone);
   sc.checksum = reinterpret_cast<uint32_t*>(base + sp.checksum);
   sc.ticket = reinterpret_cast<uint32_t*>(base + sp.ticket);
   sc.lookback = reinterpret_cast<unsigned long long*>(base + sp.lookback);
   sc.allocDone = reinterpret_cast<unsigned long long*>(base + sp.allocDone);
-  sc.ready = reinterpret_cast<uint32_t*>(base + sp.ready);
   sc.spill = base + sp.spill;
   sc.table = reinterpret_cast<uint4*>(base + sp.table);
 
-  // member table: inside the kernel parameters when it fits and the default kernels run, else one upload
+  // member table: inside the kernel parameters when it fits (the canonical encoder reads scratch), else one upload
   static thread_local InlineMembers im;
-  const bool inlined = opt.inline_members != 0 && n <= kInlineMembers && !fused && !canonical &&
-                       !(kind != kKindBytes && opt.stats_stage != 0);
+  const bool inlined = opt.inline_members != 0 && n <= kInlineMembers && !canonical;
   im.count = inlined ? n : 0u;
   if (inlined) {
-    std::memcpy(im.m, desc, descBytes);
+    std::memcpy(im.m, desc, sizeof(MemberDesc) * n);
   } else {
-    DGB_CUDA_TRY(cudaMemcpyAsync(base + sp.members, hs.upload.data(), hs.upload.size(), cudaMemcpyHostToDevice, stream));
+    DGB_CUDA_TRY(cudaMemcpyAsync(sc.members, desc, sizeof(MemberDesc) * n, cudaMemcpyHostToDevice, stream));
   }
   DGB_CUDA_TRY(cudaMemsetAsync(base + sp.zeroBegin, 0, (canonical ? sp.lookbackEnd : sp.zeroEnd) - sp.zeroBegin, stream));
 
@@ -1711,31 +1355,12 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
                          (opt.encode_wide_table > 0 || kind == DGB_BFLOAT16 || kind == DGB_FLOAT32);
   sc.wideTable = wideTable;
 
-  if (fused) {
-    // ---- one persistent launch: statistics items and encode chunks from two counters ----
-    const uint32_t statsEvery = (uint32_t)std::max(0, opt.fused_stats_every);
-    const uint32_t ti = (uint32_t)items, tc = (uint32_t)chunks;
-#define DGB_FUSED(K, WD)                                                                                          \
-  (staged ? launchFused<K, WD, true>(sc, histogram_dev, pb, checksum, n, ti, tc, slabVecs, chunkBlocks, slotWords, \
-                                     statsEvery, sp.spillWarps, outSize_dev, stream)                               \
-          : launchFused<K, WD, false>(sc, histogram_dev, pb, checksum, n, ti, tc, slabVecs, chunkBlocks, slotWords, \
-                                      statsEvery, sp.spillWarps, outSize_dev, stream))
-    switch (kind) {
-      case kKindBytes: return wideTable ? DGB_FUSED(kKindBytes, true) : DGB_FUSED(kKindBytes, false);
-      case kKindF16: return wideTable ? DGB_FUSED(kKindF16, true) : DGB_FUSED(kKindF16, false);
-      case kKindBF16: return wideTable ? DGB_FUSED(kKindBF16, true) : DGB_FUSED(kKindBF16, false);
-      case kKindF32: return wideTable ? DGB_FUSED(kKindF32, true) : DGB_FUSED(kKindF32, false);
-      default: return DGB_ERR_INVALID_ARG;
-    }
-#undef DGB_FUSED
-  }
-
-  // ---- two-kernel path: sub-batches on internal streams (the ordered canonical encoder stays on one) ----
+  // ---- sub-batches on internal streams (the ordered canonical encoder stays on one) ----
   hs.weight.resize(n);
   uint64_t totalBytes = 0;
   for (uint32_t i = 0; i < n; ++i) { hs.weight[i] = (uint64_t)desc[i].size * elemBytes; totalBytes += hs.weight[i]; }
   // byte inputs measured slightly slower when split (their stats kernel is atomics-bound, not HBM-bound)
-  const int parts = canonical ? 1 : autoParts(kind, n, totalBytes, false);
+  const int parts = canonical ? 1 : autoParts(kind, n, totalBytes);
   uint32_t bounds[kMaxParts + 1];
   splitParts(hs.weight.data(), n, parts, bounds);
   ForkGuard guard;
@@ -1757,12 +1382,7 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
     const int rc = DGB_BY_KIND(kind, residentPerSm(variant, W, smemBytes, &perSm));
     if (rc != DGB_OK) return rc;
   }
-  // option encode_k2_ctas caps the coder's CTAs per SM so that the statistics kernel of the next
-  // sub-batch finds room beside it (0 = as many as fit)
-  if (opt.encode_k2_ctas > 0) perSm = std::min(perSm, opt.encode_k2_ctas);
   const uint64_t resident = (uint64_t)perSm * sms;
-  int devForAttr = 0;
-  DGB_CUDA_TRY(cudaGetDevice(&devForAttr));
   const uint32_t spillWarpsPerPart = sp.spillWarps / (uint32_t)parts;
 
   for (int part = 0; part < parts; ++part) {
@@ -1778,34 +1398,14 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
     uint32_t partMax = 0;
     for (uint32_t i = m0; i < m1; ++i) partMax = std::max(partMax, desc[i].size);
     const uint64_t maxVecs = ((uint64_t)partMax * elemBytes) / 16u;
-    const bool stagedK1 = kind != kKindBytes && opt.stats_stage != 0;
-    const uint32_t slabVecsK1 = stagedK1 ? std::min<uint32_t>(slabVecs, (uint32_t)std::max(1, opt.stats_stage_kb) * 64u) : slabVecs;
-    uint32_t gridY = (uint32_t)std::max<uint64_t>(1, (maxVecs + slabVecsK1 - 1) / slabVecsK1);
-    if (!stagedK1) {
-      // enough CTAs to fill the machine a few times, never more than the slabs
-      const uint32_t wantY = std::max(1u, (uint32_t)(std::max(1, opt.hist_ctas_per_sm) * sms) / (m1 - m0));
-      gridY = std::min(gridY, wantY);
-    }
+    uint32_t gridY = (uint32_t)std::max<uint64_t>(1, (maxVecs + slabVecs - 1) / slabVecs);
+    // enough CTAs to fill the machine a few times, never more than the slabs
+    const uint32_t wantY = std::max(1u, (uint32_t)(std::max(1, opt.hist_ctas_per_sm) * sms) / (m1 - m0));
+    gridY = std::min(gridY, wantY);
     gridY = std::min(gridY, 65535u);
     dim3 grid1(m1 - m0, gridY);
     timerBegin(kSlotStats, ps);
-    if (stagedK1 && gridY * (uint64_t)slabVecsK1 >= maxVecs) {
-      const size_t stageBytes = (size_t)slabVecsK1 * 16u;
-      static thread_local int stagedDev = -1;
-      if (stagedDev != devForAttr) {
-        DGB_CUDA_TRY(cudaFuncSetAttribute(statsFloatStagedKernel<DGB_FLOAT16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024));
-        DGB_CUDA_TRY(cudaFuncSetAttribute(statsFloatStagedKernel<DGB_BFLOAT16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024));
-        DGB_CUDA_TRY(cudaFuncSetAttribute(statsFloatStagedKernel<DGB_FLOAT32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024));
-        stagedDev = devForAttr;
-      }
-      if (kind == kKindF16) {
-        statsFloatStagedKernel<DGB_FLOAT16><<<grid1, kStatsThreads, stageBytes, ps>>>(sc, pb, checksum, slabVecsK1, m0, outSize_dev);
-      } else if (kind == kKindBF16) {
-        statsFloatStagedKernel<DGB_BFLOAT16><<<grid1, kStatsThreads, stageBytes, ps>>>(sc, pb, checksum, slabVecsK1, m0, outSize_dev);
-      } else {
-        statsFloatStagedKernel<DGB_FLOAT32><<<grid1, kStatsThreads, stageBytes, ps>>>(sc, pb, checksum, slabVecsK1, m0, outSize_dev);
-      }
-    } else if (kind == kKindBytes) {
+    if (kind == kKindBytes) {
       statsBytesKernel<<<grid1, kStatsThreads, 0, ps>>>(sc, im, histogram_dev, pb, checksum, slabVecs, m0, outSize_dev);
     } else if (kind == kKindF16) {
       statsFloatKernel<DGB_FLOAT16><<<grid1, kStatsThreads, 0, ps>>>(sc, im, pb, checksum, slabVecs, m0, outSize_dev);
@@ -1827,7 +1427,8 @@ int encodeBatch(int kind, void* temp, size_t tempBytes, int pb, bool checksum, u
       if (canonical) {
         grid2 = std::min<uint32_t>(divUp(totalTickets, W), (uint32_t)resident);
       } else {
-        // one resident wave, equal rounds per warp (see launchDecode)
+        // one resident wave, every warp gets the same number of blocks (rounds) when the batch is large,
+        // so no warp idles at the end waiting for a neighbour's extra block
         const uint64_t rounds = std::max<uint64_t>(1, (partBlocks + resident * W - 1) / (resident * W));
         const uint64_t want = ((uint64_t)partBlocks + W * rounds - 1) / (W * rounds);
         grid2 = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(want, resident));

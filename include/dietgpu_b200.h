@@ -212,7 +212,8 @@ int dgb_set_thread_option(const char* name, int value);
 int dgb_clear_thread_options(void);
 /* With option "timing" = 1 every kernel launch is bracketed by CUDA events on the caller's
  * stream; this returns (and resets) the summed durations in ms and launch counts per kernel:
- * slot 0 stats (K1), 1 encode (K2), 2 plan, 3 decode, 4 checksum, 5 fused encode, 6 archive mover.  Synchronises the device. */
+ * slot 0 stats (K1), 1 encode (K2), 2 retired (always 0), 3 decode, 4 checksum, 5 retired (always 0), 6 archive mover.
+ * Synchronises the device. */
 int dgb_kernel_times(float* ms, int* counts, int nslots);
 
 #ifdef __cplusplus

@@ -44,7 +44,7 @@ def test_temp_sizes_are_sane():
     assert L.dgb_float_compress_temp_bytes(capi.FLOAT16, 3, 10000) < (1 << 20)
 
 
-def test_error_codes_without_gpu():
+def test_error_codes_and_option_names_without_gpu():
     L = capi.lib()
     assert capi.error_string(capi.OK) == "ok"
     assert "temporary" in capi.error_string(capi.ERR_TEMP_TOO_SMALL)
@@ -58,8 +58,14 @@ def test_error_codes_without_gpu():
     assert L.dgb_float_compress_pointer(None, 0, 9, 10, 0, 1, one, sz, one, None, None) == capi.ERR_INVALID_ARG
     assert L.dgb_ans_encode_pointer(None, 0, 10, 0, 1, one, sz, None, one, None, None) == capi.ERR_TEMP_TOO_SMALL
     assert L.dgb_set_option(b"no_such_option", 1) == capi.ERR_INVALID_ARG
-    capi.set_option("decode_fused", 1)
-    assert capi.get_option("decode_fused") == 1
+    capi.set_option("inline_members", 1)
+    assert capi.get_option("inline_members") == 1
+    # retired kernel variants: their options are unknown names now
+    for name in ("encode_fused", "decode_fused", "fused_stage", "fused_stats_every", "fused_chunk_blocks",
+                 "stats_stage", "stats_stage_kb", "encode_k2_ctas", "first_part_pct", "last_part_pct"):
+        assert L.dgb_set_option(name.encode(), 1) == capi.ERR_INVALID_ARG, name
+        v = C.c_int(0)
+        assert L.dgb_get_option(name.encode(), C.byref(v)) == capi.ERR_INVALID_ARG, name
 
 
 def test_product_does_not_import_oracle():

@@ -459,33 +459,22 @@ def test_encoder_table_formats():
         capi.set_option("encode_wide_table", -1)
 
 
-def test_kernel_variants_agree():
-    # every tuning variant produces identical results: single-launch vs two-kernel paths in both
-    # directions, chunk sizes, statistics-CTA share, warps per CTA, canonical packing
+def test_tuning_options_agree():
+    # every tuning variant produces identical results: warps per CTA in both directions, canonical
+    # packing, member table in the kernel parameters or in scratch
     from dietgpu_b200 import capi
 
     a = [zipf_bytes(300000, 1.1, 5), exp_bytes(4097, 50, 6), zipf_bytes(1, 1.0, 7), np.zeros(0, np.uint8)]
     f = [normal_words(50000 + 13 * i, "bf16", i) for i in range(5)]
-    names = ("encode_fused", "decode_fused", "fused_chunk_blocks", "fused_stats_every", "fused_stage",
-             "encode_warps", "encode_canonical", "inline_members", "decode_warps")
+    names = ("encode_warps", "encode_canonical", "inline_members", "decode_warps")
     defaults = {k: capi.get_option(k) for k in names}
     variants = [
-        dict(encode_fused=0, decode_fused=0),
-        dict(encode_fused=1, decode_fused=0),
-        dict(encode_fused=0, decode_fused=1),
-        dict(encode_fused=1, fused_chunk_blocks=2),
-        dict(fused_chunk_blocks=1),
-        dict(fused_chunk_blocks=3, fused_stage=0),
-        dict(fused_chunk_blocks=64),
-        dict(fused_stats_every=0),
-        dict(fused_stats_every=1),
-        dict(encode_fused=0, encode_warps=2),
-        dict(encode_fused=0, encode_warps=4),
+        {},
+        dict(encode_warps=2),
+        dict(encode_warps=4),
         dict(encode_canonical=1),
-        dict(encode_canonical=1, decode_fused=0),
         dict(decode_warps=20),  # byte archives: 20-warp decoder CTAs (auto only for long members)
         dict(decode_warps=8),
-        dict(decode_warps=4),
         dict(inline_members=0),  # member table uploaded to scratch instead of travelling in the kernel parameters
     ]
     try:

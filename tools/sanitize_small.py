@@ -28,8 +28,6 @@ def bytes_(n, off=0):
 VARIANTS = [
     {},
     {"encode_canonical": 1},
-    {"encode_fused": 1},
-    {"decode_fused": 0},
     {"inline_members": 0},
     {"decode_warps": 20},
     {"encode_warps": 2, "decode_slot_words": 512, "encode_slot_words": 512},

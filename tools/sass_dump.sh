@@ -14,7 +14,6 @@ dump encode 'statsFloatKernelILi2EE' stats_bf16
 dump encode 'statsBytesKernelE' stats_bytes
 dump encode 'encodeKernelFastILb0ELi0' encode_bytes_packed
 dump encode 'encodeKernelFastILb1ELi2' encode_bf16_wide
-dump encode 'encodeFusedKernelILi2ELb1ELb1' encode_fused_bf16_staged
 dump decode 'decodeFusedKernelILi2ELi10ELi8' decode_bf16_pb10
 dump decode 'decodeFusedKernelILi0ELi10ELi8' decode_bytes_pb10
 {

@@ -32,8 +32,8 @@ for v in variants:
         codec.encode(); codec.decode()
     kt = capi.kernel_times(); capi.set_option("timing", 0)
     ms = {k: kt[k][0] / max(kt[k][1], 1) for k in kt}
-    enc = ms["stats"] + ms["encode"]; dec = ms["plan"] + ms["decode"]
+    enc = ms["stats"] + ms["encode"]; dec = ms["decode"]
     print(f"{wl} [{v}] ok={ok} ratio={sum(hs)/ub:.4f} stats={ms['stats']*1e3:.1f}us encode={ms['encode']*1e3:.1f}us "
-          f"plan={ms['plan']*1e3:.1f}us decode={ms['decode']*1e3:.1f}us | enc {ub/enc/1e6:.0f} GB/s dec {ub/dec/1e6:.0f} GB/s (kernel-only)", flush=True)
+          f"decode={ms['decode']*1e3:.1f}us | enc {ub/enc/1e6:.0f} GB/s dec {ub/dec/1e6:.0f} GB/s (kernel-only)", flush=True)
     for k in opts:
         pass
